@@ -22,11 +22,12 @@ ON_INFEASIBLE = {"hold": 0, "respawn": 1}
 PRECISION = {"fp64": 0, "fp32": 1}
 HOT_PATH = {"auto": 0, "cta": 1}
 GATE = {"off": 0, "schedule": 1, "detect": 2}
+BODY = {"model": 1, "plant": 2, "both": 3}
 
 # every symbol include/hmpc.h declares (tests/test_abi.py checks the .so exports all of them)
 SYMBOLS = [
     "hmpc_default_config", "hmpc_create", "hmpc_destroy", "hmpc_set_stream", "hmpc_synchronize",
-    "hmpc_set_gains", "hmpc_convert", "hmpc_rk4", "hmpc_linearize", "hmpc_condense", "hmpc_solve",
+    "hmpc_set_gains", "hmpc_set_body_params", "hmpc_convert", "hmpc_rk4", "hmpc_linearize", "hmpc_condense", "hmpc_solve",
     "hmpc_rollout", "hmpc_plan_set", "hmpc_plan_tables", "hmpc_rollout_planned", "hmpc_set_contact_gate", "hmpc_solve_stats", "hmpc_set_timing", "hmpc_kernel_times", "hmpc_tick_times", "hmpc_launch_count", "hmpc_hot_path_info", "hmpc_measure_fp64_peak", "hmpc_last_error",
     "hmpc_abi_version",
 ]
@@ -81,6 +82,7 @@ def load():
     lib.hmpc_set_stream.argtypes = [vp, vp]
     lib.hmpc_synchronize.argtypes = [vp]
     lib.hmpc_set_gains.argtypes = [vp, vp, vp]
+    lib.hmpc_set_body_params.argtypes = [vp, i32, vp, vp, vp, vp, vp]
     lib.hmpc_convert.argtypes = [vp, vp, vp]
     lib.hmpc_rk4.argtypes = [vp, vp, vp, vp, i32, vp]
     lib.hmpc_linearize.argtypes = [vp, vp, vp, vp, vp]

@@ -110,6 +110,22 @@ class BatchMpc:
             self._chk(Rdiag, (6, self.B))
         _lib.check(self.lib.hmpc_set_gains(self._h, _ptr(Qdiag), _ptr(Rdiag)))
 
+    def set_body_params(self, which="both", m=None, J=None, Jinv=None, rh=None, mu=None):
+        """Per-hopper body (include/hmpc.h: hmpc_set_body_params).  which: "model" (what the MPC plans with: m, Jinv,
+        rh, mu), "plant" (what rk4 / the rollouts integrate: m, J, Jinv, rh) or "both".  Tensors: m (B,), J and Jinv
+        (3, 3, B), rh (3, B), mu (B,); None keeps the config's scalar for every hopper, all None resets the target.
+        Jinv is computed from J when only J is given."""
+        B = self.B
+        if which not in _lib.BODY:
+            raise ValueError(f"which must be one of {sorted(_lib.BODY)}, got {which!r}")
+        for t, shape in ((m, (B,)), (J, (3, 3, B)), (Jinv, (3, 3, B)), (rh, (3, B)), (mu, (B,))):
+            if t is not None:
+                self._chk(t, shape)
+        if J is not None and Jinv is None and which != "model":
+            Jinv = soa(torch.linalg.inv(aos(J)))
+        _lib.check(self.lib.hmpc_set_body_params(self._h, _lib.BODY[which], _ptr(m), _ptr(J), _ptr(Jinv), _ptr(rh),
+                                                 _ptr(mu)))
+
     def convert(self, X):
         self._chk(X, (13, self.B))
         x = self.empty(12, self.B)

@@ -109,13 +109,21 @@ struct hmpc_handle {
     int gate_max_tick = 0;
     double leg_max = 0.0;
     int32_t* n_defer = nullptr;   // [1] accumulated deferrals of the most recent solve / rollout
+    // per-hopper bodies (hmpc_set_body_params), allocated on the first call; used while the flag is set
+    double* body_model = nullptr;   // [kBodyModel][B]  QpConst::body
+    double* body_plant = nullptr;   // [kBodyPlant][B]  SimConst::body
+    bool model_on = false, plant_on = false;
+    int* body_bad = nullptr;        // [1] first hopper with invalid values (body_check_kernel)
 };
 
 namespace hmpc {
 
 // ------------------------------------------------------------------------------------------------
 // K3: simulator.  X [13][B] in/out; U [6][B]; pfa/pfb [3][B] footstep before/after the switch step.
+// PLANT: every hopper integrates its own body (c.body set); the uniform build keeps the body in the kernel's constant
+// parameters and needs no registers for it.
 // ------------------------------------------------------------------------------------------------
+template <bool PLANT>
 __global__ void __launch_bounds__(128)
 sim_kernel(SimConst c, int B, double* __restrict__ X, const double* __restrict__ U,
            const double* __restrict__ pfa, const double* __restrict__ pfb,
@@ -148,7 +156,8 @@ sim_kernel(SimConst c, int B, double* __restrict__ X, const double* __restrict__
         mat3T_vec(R, xr + 6, Xl + 7);
         Xl[10] = Xl[11] = Xl[12] = 0.0;
     } else {
-        sim_tick(c, gt.mode, gate_bits_of(gt, b), gt.leg_max2, Xl, Ul, pa, pb, s, nsteps, Xsteps, (size_t)B, b);
+        if (PLANT) sim_tick(plant_body(c, b, B), gt.mode, gate_bits_of(gt, b), gt.leg_max2, Xl, Ul, pa, pb, s, nsteps, Xsteps, (size_t)B, b);
+        else sim_tick(c, gt.mode, gate_bits_of(gt, b), gt.leg_max2, Xl, Ul, pa, pb, s, nsteps, Xsteps, (size_t)B, b);
     }
 #pragma unroll
     for (int i = 0; i < 13; ++i) X[(size_t)i * B + b] = Xl[i];
@@ -188,13 +197,14 @@ __global__ void linearize_kernel(QpConst c, int B, const double* __restrict__ x_
     carve(w, smem, c.N);
     const int N = c.N, tid = threadIdx.x, T = blockDim.x, b = blockIdx.x;
     for (int i = tid; i < 3 * N; i += T) w.pfw[i] = pf[(size_t)i * B + b];
+    stage_body(c, w, b, B);
     for (int k = tid; k < N; k += T) {
         const size_t o = (size_t)k * 12;
         w.gp[4 * k] = x_guess[(o + 0) * B + b]; w.gp[4 * k + 1] = x_guess[(o + 1) * B + b];
         w.gp[4 * k + 2] = x_guess[(o + 2) * B + b]; w.gp[4 * k + 3] = x_guess[(o + 5) * B + b];
     }
     __syncthreads();
-    for (int k = tid; k < N; k += T) linearize_stage(c, k, w);
+    for (int k = tid; k < N; k += T) linearize_stage(c, SmemBody{w.red}, k, w);
     __syncthreads();
     for (int e = tid; e < N * 144; e += T) {
         const int k = e / 144, r = (e % 144) / 12, cc = e % 12;
@@ -236,12 +246,41 @@ __global__ void condense_kernel(QpConst c, int B, int mats_in_smem, double* __re
             w.gp[4 * k + 2] = x_guess[(o + 2) * B + b]; w.gp[4 * k + 3] = x_guess[(o + 5) * B + b];
         }
         __syncthreads();
-        const int inf = condense(c, w, x_ref + b, (size_t)B);
+        const int inf = condense_hopper(c, w, b, B, x_ref + b, (size_t)B);
         if (infeasible && tid == 0) infeasible[b] = inf;
         for (int e = tid; e < n * n; e += T) H[(size_t)e * B + b] = sym_at(w.H, n, e / n, e % n);
         for (int i = tid; i < n; i += T) g[(size_t)i * B + b] = w.g[i];
         for (int r = tid; r < m; r += T) { lo[(size_t)r * B + b] = w.lo[r]; hi[(size_t)r * B + b] = w.hi[r]; }
     }
+}
+
+// hmpc_set_body_params: *bad = min over the hoppers whose given values are not finite, or m <= 0, or mu < 0
+__global__ void body_check_kernel(int B, const double* __restrict__ m, const double* __restrict__ J,
+                                  const double* __restrict__ Jinv, const double* __restrict__ rh,
+                                  const double* __restrict__ mu, int* __restrict__ bad) {
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return;
+    const size_t Bs = (size_t)B;
+    bool ok = true;
+    if (m) ok = ok && isfinite(m[b]) && m[b] > 0.0;
+    if (mu) ok = ok && isfinite(mu[b]) && mu[b] >= 0.0;
+    for (int i = 0; i < 9; ++i) {
+        if (J) ok = ok && isfinite(J[i * Bs + b]);
+        if (Jinv) ok = ok && isfinite(Jinv[i * Bs + b]);
+        if (i < 3 && rh) ok = ok && isfinite(rh[i * Bs + b]);
+    }
+    if (!ok) atomicMin(bad, b);
+}
+// rows of a body array that take the handle's scalar for every hopper (bit r of mask: row r = v[r])
+struct BodyFill {
+    double v[kBodyPlant];
+    uint32_t mask;
+};
+__global__ void body_fill_kernel(int B, double* __restrict__ dst, BodyFill f) {
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return;
+    for (int r = 0; r < kBodyPlant; ++r)
+        if ((f.mask >> r) & 1u) dst[(size_t)r * B + b] = f.v[r];
 }
 
 // FP64 FMA peak: 8 independent accumulator chains per thread, no memory traffic in the loop.
@@ -305,6 +344,23 @@ hmpc::SimConst make_sim_const(const hmpc_config& cfg) {
     for (int i = 0; i < 9; ++i) { s.J[i] = cfg.J[i]; s.Jinv[i] = cfg.Jinv[i]; }
     for (int i = 0; i < 3; ++i) s.rh[i] = cfg.rh[i];
     return s;
+}
+
+hmpc::QpConst qp_const(const hmpc_handle* h) {
+    hmpc::QpConst c = make_qp_const(h->cfg);
+    c.body = h->model_on ? h->body_model : nullptr;
+    return c;
+}
+hmpc::SimConst sim_const(const hmpc_handle* h) {
+    hmpc::SimConst s = make_sim_const(h->cfg);
+    s.body = h->plant_on ? h->body_plant : nullptr;
+    return s;
+}
+// the simulator kernel, specialised on whether the hoppers carry their own plant body
+template <class... Args>
+void launch_sim(const hmpc::SimConst& sc, int grid, cudaStream_t st, Args... args) {
+    if (sc.body) hmpc::sim_kernel<true><<<grid, 128, 0, st>>>(sc, args...);
+    else hmpc::sim_kernel<false><<<grid, 128, 0, st>>>(sc, args...);
 }
 
 int check_handle(hmpc_handle* h) {
@@ -592,6 +648,7 @@ int hmpc_destroy(hmpc_handle* h) {
     cudaFree(h->gate_glob);
     cudaFree(h->prep); cudaFree(h->prep_flag); cudaFree(h->defer_list); cudaFree(h->n_defer);
     cudaFree(h->work_order); cudaFree(h->order_cnt); cudaFree(h->warm); cudaFree(h->warm_ok);
+    cudaFree(h->body_model); cudaFree(h->body_plant); cudaFree(h->body_bad);
     for (cudaEvent_t e : h->ev) cudaEventDestroy(e);
     delete h;
     return HMPC_OK;
@@ -617,6 +674,71 @@ int hmpc_set_gains(hmpc_handle* h, const double* Qdiag, const double* Rdiag) {
     return HMPC_OK;
 }
 
+int hmpc_set_body_params(hmpc_handle* h, int which, const double* m, const double* J, const double* Jinv, const double* rh,
+                         const double* mu) {
+    if (int rc = check_handle(h)) return rc;
+    if (which != HMPC_BODY_MODEL && which != HMPC_BODY_PLANT && which != HMPC_BODY_BOTH)
+        return fail(HMPC_ERR_BAD_ARG, "which must be HMPC_BODY_MODEL, HMPC_BODY_PLANT or HMPC_BODY_BOTH");
+    if (J && which == HMPC_BODY_MODEL) return fail(HMPC_ERR_BAD_ARG, "J is a plant quantity: the MPC model uses Jinv only");
+    if (mu && which == HMPC_BODY_PLANT) return fail(HMPC_ERR_BAD_ARG, "mu is a model quantity: the simulator has no friction");
+    const bool model = which & HMPC_BODY_MODEL, plant = which & HMPC_BODY_PLANT;
+    if (!m && !J && !Jinv && !rh && !mu) {          // back to the config's scalars for every hopper
+        if (model) h->model_on = false;
+        if (plant) h->plant_on = false;
+        return HMPC_OK;
+    }
+    const int Bi = h->cfg.batch, grid = (Bi + 127) / 128;
+    const size_t B = (size_t)Bi;
+    if (!h->body_bad) HMPC_CUDA(cudaMalloc((void**)&h->body_bad, sizeof(int)));
+    if (model && !h->body_model) HMPC_CUDA(cudaMalloc((void**)&h->body_model, hmpc::kBodyModel * B * 8));
+    if (plant && !h->body_plant) HMPC_CUDA(cudaMalloc((void**)&h->body_plant, hmpc::kBodyPlant * B * 8));
+    // validate what was given before anything is replaced: a rejected call leaves the handle as it was
+    int bad = INT32_MAX;
+    HMPC_CUDA(cudaMemcpyAsync(h->body_bad, &bad, sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    hmpc::body_check_kernel<<<grid, 128, 0, h->stream>>>(Bi, m, J, Jinv, rh, mu, h->body_bad);
+    ++h->launches;
+    HMPC_CUDA(cudaGetLastError());
+    HMPC_CUDA(cudaMemcpyAsync(&bad, h->body_bad, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    HMPC_CUDA(cudaStreamSynchronize(h->stream));
+    if (bad != INT32_MAX)
+        return fail(HMPC_ERR_BAD_ARG, "hmpc_set_body_params: hopper " + std::to_string(bad) +
+                                          " has a non-finite value, m <= 0 or mu < 0");
+    // one target: rows of the given arrays copied, the other rows filled with the config's scalars
+    auto set = [&](double* dst, int r_m, int r_rh, int r_J, int r_Jinv, int r_mu) -> int {
+        hmpc::BodyFill f;
+        f.mask = 0;
+        auto row = [&](int r0, int nr, const double* src, const double* scal) -> int {
+            if (r0 < 0) return HMPC_OK;
+            if (src) {
+                HMPC_CUDA(cudaMemcpyAsync(dst + (size_t)r0 * B, src, (size_t)nr * B * 8, cudaMemcpyDeviceToDevice, h->stream));
+            } else {
+                for (int i = 0; i < nr; ++i) { f.v[r0 + i] = scal[i]; f.mask |= 1u << (r0 + i); }
+            }
+            return HMPC_OK;
+        };
+        int rc;
+        if ((rc = row(r_m, 1, m, &h->cfg.m)) || (rc = row(r_rh, 3, rh, h->cfg.rh)) || (rc = row(r_J, 9, J, h->cfg.J)) ||
+            (rc = row(r_Jinv, 9, Jinv, h->cfg.Jinv)) || (rc = row(r_mu, 1, mu, &h->cfg.mu)))
+            return rc;
+        if (f.mask) {
+            hmpc::body_fill_kernel<<<grid, 128, 0, h->stream>>>(Bi, dst, f);
+            ++h->launches;
+            HMPC_CUDA(cudaGetLastError());
+        }
+        return HMPC_OK;
+    };
+    // row order: QpConst::body = m, mu, rh, Jinv (hmpc::Body); SimConst::body = m, rh, J, Jinv (hmpc::plant_body)
+    if (model) {
+        if (int rc = set(h->body_model, 0, 2, -1, 5, 1)) return rc;
+        h->model_on = true;
+    }
+    if (plant) {
+        if (int rc = set(h->body_plant, 0, 1, 4, 13, -1)) return rc;
+        h->plant_on = true;
+    }
+    return HMPC_OK;
+}
+
 int hmpc_convert(hmpc_handle* h, const double* X, double* x) {
     if (int rc = check_handle(h)) return rc;
     if (!X || !x) return fail(HMPC_ERR_BAD_ARG, "null array");
@@ -631,9 +753,9 @@ int hmpc_rk4(hmpc_handle* h, double* X, const double* U, const double* pf, int n
     if (int rc = check_handle(h)) return rc;
     if (!X || !U || !pf || nsteps < 0) return fail(HMPC_ERR_BAD_ARG, "bad argument");
     const int B = h->cfg.batch;
-    hmpc::sim_kernel<<<(B + 127) / 128, 128, 0, h->stream>>>(make_sim_const(h->cfg), B, X, U, pf, nullptr,
-                                                              nullptr, nsteps, nullptr, nullptr, nullptr, X_steps, nullptr, nullptr,
-                                                              hmpc::SimGate{HMPC_GATE_OFF, nullptr, nullptr, nullptr, 0, 0, 0.0});
+    launch_sim(sim_const(h), (B + 127) / 128, h->stream, B, X, U, pf, (const double*)nullptr, (const uint8_t*)nullptr, nsteps,
+               (double*)nullptr, (double*)nullptr, (double*)nullptr, X_steps, (const int32_t*)nullptr, (const double*)nullptr,
+               hmpc::SimGate{HMPC_GATE_OFF, nullptr, nullptr, nullptr, 0, 0, 0.0});
     ++h->launches;
     HMPC_CUDA(cudaGetLastError());
     return HMPC_OK;
@@ -643,7 +765,7 @@ int hmpc_linearize(hmpc_handle* h, const double* x_guess, const double* pf, doub
     if (int rc = check_handle(h)) return rc;
     if (!x_guess || !pf || !Ad || !Bd) return fail(HMPC_ERR_BAD_ARG, "null array");
     const size_t vec_bytes = ((hmpc::work_vec_doubles(h->cfg.N) + 1) & ~(size_t)1) * 8;
-    hmpc::linearize_kernel<<<h->cfg.batch, 128, vec_bytes, h->stream>>>(make_qp_const(h->cfg), h->cfg.batch,
+    hmpc::linearize_kernel<<<h->cfg.batch, 128, vec_bytes, h->stream>>>(qp_const(h), h->cfg.batch,
                                                                         x_guess, pf, Ad, Bd);
     ++h->launches;
     HMPC_CUDA(cudaGetLastError());
@@ -657,7 +779,7 @@ int hmpc_condense(hmpc_handle* h, const double* x_in, const double* x_guess, con
     if (!x_in || !x_guess || !x_ref || !pf || !Cbits || !H || !g || !lo || !hi)
         return fail(HMPC_ERR_BAD_ARG, "null array");
     hmpc::condense_kernel<<<h->mpc_grid, h->mpc_threads, h->mpc_smem, h->stream>>>(
-        make_qp_const(h->cfg), h->cfg.batch, h->mats_in_smem ? 1 : 0, h->ws, x_in, x_guess, x_ref, pf, Cbits,
+        qp_const(h), h->cfg.batch, h->mats_in_smem ? 1 : 0, h->ws, x_in, x_guess, x_ref, pf, Cbits,
         h->Qd, h->Rd, H, g, lo, hi, infeasible);
     ++h->launches;
     HMPC_CUDA(cudaGetLastError());
@@ -769,7 +891,7 @@ int hmpc_solve(hmpc_handle* h, const double* x_in, const double* x_ref, const do
     hmpc::MpcIo io = make_io(h, x_in, x_ref, pf, Cbits, init ? 1 : 0, 0, U, Xsol, nullptr, status, iters);
     io.respawn = 0;   // per-hopper re-initialisation only exists inside hmpc_rollout
     HMPC_CUDA(cudaMemsetAsync(h->n_defer, 0, 4, h->stream));
-    HMPC_CUDA(launch_mpc(h, make_qp_const(h->cfg), io));
+    HMPC_CUDA(launch_mpc(h, qp_const(h), io));
     return HMPC_OK;
 }
 
@@ -800,8 +922,8 @@ int rollout_impl(hmpc_handle* h, bool planned, double* X, const double* xref_tab
     if (h->gate_mode == HMPC_GATE_SCHEDULE && (planned ? !h->gate_glob : !h->gate_tab))
         return fail(HMPC_ERR_BAD_ARG, planned ? "HMPC_GATE_SCHEDULE: hmpc_set_contact_gate was given no gate_glob for hmpc_rollout_planned"
                                               : "HMPC_GATE_SCHEDULE: hmpc_set_contact_gate was given no gate_tab for hmpc_rollout");
-    const hmpc::QpConst qc = make_qp_const(h->cfg);
-    const hmpc::SimConst sc = make_sim_const(h->cfg);
+    const hmpc::QpConst qc = qp_const(h);
+    const hmpc::SimConst sc = sim_const(h);
     const int sim_grid = (Bi + 127) / 128;
     const bool respawn = h->cfg.on_infeasible == HMPC_INFEASIBLE_RESPAWN;
     // x_in for the first tick; afterwards sim_kernel emits it fused with the integration
@@ -831,10 +953,10 @@ int rollout_impl(hmpc_handle* h, bool planned, double* X, const double* xref_tab
         if (h->timing) HMPC_CUDA(cudaEventRecord(h->ev[3 * t], h->stream));
         HMPC_CUDA(launch_mpc(h, qc, io));
         if (h->timing) HMPC_CUDA(cudaEventRecord(h->ev[3 * t + 1], h->stream));
-        hmpc::sim_kernel<<<sim_grid, 128, 0, h->stream>>>(
-            sc, Bi, X, h->U0, pf, pf + 3 * B, sw, h->cfg.mpc_factor, h->xin,
+        launch_sim(sc, sim_grid, h->stream,
+            Bi, X, (const double*)h->U0, pf, pf + 3 * B, sw, h->cfg.mpc_factor, h->xin,
             X_log ? X_log + (size_t)(t + 1) * 13 * B : nullptr, U_log ? U_log + (size_t)t * 6 * B : nullptr,
-            nullptr, respawn ? h->st_tick : nullptr, respawn ? xr + 12 * B : nullptr, gate);
+            (double*)nullptr, respawn ? (const int32_t*)h->st_tick : nullptr, respawn ? xr + 12 * B : nullptr, gate);
         if (h->timing) HMPC_CUDA(cudaEventRecord(h->ev[3 * t + 2], h->stream));
         ++h->launches;
     }

@@ -42,7 +42,9 @@ mpc_kernel(QpConst c, int B, int sm_count, double* __restrict__ ws, int* __restr
         const int i = s_next;
         if (i >= count) break;
         const int e = list ? list[i] : work_item(c, i, count);     // bit 30: the warp kernel's active-set refinement already gave up
-        mpc_hopper<WITH_ADMM>(c, w, sys, A, e & ~(1 << 30), B, io, (e >> 30) & 1);
+        const int b = e & ~(1 << 30);
+        if (c.body) A.mu = c.body[(size_t)B + b];                  // the hopper's friction coefficient (model_body)
+        mpc_hopper<WITH_ADMM>(c, w, sys, A, b, B, io, (e >> 30) & 1);
     }
 }
 

@@ -98,6 +98,8 @@ struct MpcIo {
 
 // One hopper b of a batch of B.  All threads of the CTA call this together.
 // WITH_ADMM = false compiles the OSQP-style ADMM branch out (smaller kernel for the default exact solver)
+// A.mu must be hopper b's friction coefficient (model_body).  The caller sets it on its own A: a modified by-value copy
+// here made the compiler lose the shared-memory address space of A's arrays (generic loads instead of LDS).
 template <bool WITH_ADMM, class Sys>
 __device__ inline void mpc_hopper(const QpConst& c, Work& w, Sys& sys, const AOp& A, int b, int B, const MpcIo& io,
                                   int skip_warm = 0) {
@@ -136,7 +138,7 @@ __device__ inline void mpc_hopper(const QpConst& c, Work& w, Sys& sys, const AOp
         __syncthreads();
         PH_ADD(1, ph_all);
         PH_T0(ph_c);
-        const int infeasible = condense(c, w, io.x_ref + b, (size_t)B);
+        const int infeasible = condense_hopper(c, w, b, B, io.x_ref + b, (size_t)B);
         PH_ADD(2, ph_c);
         PH_T0(ph_sv);
         sys.flops += c.condense_flops;

@@ -68,11 +68,57 @@ struct QpConst {
     // optional second stage of that map (lock-step solve kernel only): a permutation of the hoppers that puts equal
     // contact schedules next to each other (hmpc_api.cu: order_* kernels), or null
     const int* work_order;
+    // per-hopper model body (hmpc_set_body_params), [kBodyModel][B] in Body's field order, or null: every hopper plans
+    // with the scalars m, mu, rh, Jinv above (the default path then does no extra loads)
+    const double* body = nullptr;
 };
 __device__ __forceinline__ int work_item(const QpConst& c, int i, int B) {
     const int t = (int)(((long long)i * c.work_mul + c.work_add) % B);
     return c.work_order ? c.work_order[t] : t;
 }
+
+// The body the MPC plans with for hopper b (the arguments of Mpc.__init__ minus g, mpc_cvx_euler_3f.py:12-39).
+// Always indexed by hopper, never by work ticket.
+struct Body {
+    double m, mu, rh[3], Jinv[9];
+};
+constexpr int kBodyModel = 14;        // doubles per hopper of QpConst::body
+__device__ __forceinline__ Body scalar_body(const QpConst& c) {
+    Body bd;
+    bd.m = c.m; bd.mu = c.mu;
+#pragma unroll
+    for (int i = 0; i < 3; ++i) bd.rh[i] = c.rh[i];
+#pragma unroll
+    for (int i = 0; i < 9; ++i) bd.Jinv[i] = c.Jinv[i];
+    return bd;
+}
+__device__ __forceinline__ Body model_body(const QpConst& c, int b, int B) {
+    if (!c.body) return scalar_body(c);
+    Body bd;
+    {
+        const double* p = c.body + b;
+        const size_t Bs = (size_t)B;
+        bd.m = p[0]; bd.mu = p[Bs];
+#pragma unroll
+        for (int i = 0; i < 3; ++i) bd.rh[i] = p[(2 + i) * Bs];
+#pragma unroll
+        for (int i = 0; i < 9; ++i) bd.Jinv[i] = p[(5 + i) * Bs];
+    }
+    return bd;
+}
+// The CTA kernel's condensing reads the body through one of two sources, chosen per hopper on QpConst::body: the
+// QpConst itself (its scalars) or a shared-memory copy of hopper b's body (condense_hopper: the model array's column,
+// or the scalars when none is set).  Neither keeps the body in registers across the condensing: the 128-register
+// builds of that kernel have no room for it.
+struct SmemBody {
+    const double* s;   // [kBodyModel] in QpConst::body's row order
+};
+__device__ __forceinline__ double body_m(const QpConst& c) { return c.m; }
+__device__ __forceinline__ double body_rh(const QpConst& c, int i) { return c.rh[i]; }
+__device__ __forceinline__ double body_Jinv(const QpConst& c, int i) { return c.Jinv[i]; }
+__device__ __forceinline__ double body_m(const SmemBody& h) { return h.s[0]; }
+__device__ __forceinline__ double body_rh(const SmemBody& h, int i) { return h.s[2 + i]; }
+__device__ __forceinline__ double body_Jinv(const SmemBody& h, int i) { return h.s[5 + i]; }
 
 // ------------------------------------------------------------------------------------------------
 // shared-memory carve-up (all doubles unless noted)
@@ -307,7 +353,8 @@ struct AOp {
 // ------------------------------------------------------------------------------------------------
 // linearisation of one stage (gen_dt_dynamics); thread k handles stage k
 // ------------------------------------------------------------------------------------------------
-__device__ inline void linearize_stage(const QpConst& c, int k, Work& w) {
+template <class Bd>   // QpConst (the scalars) or SmemBody
+__device__ inline void linearize_stage(const QpConst& c, const Bd& bd, int k, Work& w) {
     const double psi = w.gp[4 * k + 3];
     double sn, cs;
     sincos(psi, &sn, &cs);
@@ -317,13 +364,13 @@ __device__ inline void linearize_stage(const QpConst& c, int k, Work& w) {
                          w.pfw[3 * k + 2] - w.gp[4 * k + 2]};
     double rf[3];
     mat3_vec(Rz, d, rf);
-    rf[0] += c.rh[0]; rf[1] += c.rh[1]; rf[2] += c.rh[2];
+    rf[0] += body_rh(bd, 0); rf[1] += body_rh(bd, 1); rf[2] += body_rh(bd, 2);
     // Jw = Rz Jinv Rz^T
     double T1[9], Jw[9];
     for (int i = 0; i < 3; ++i)
         for (int j = 0; j < 3; ++j) {
             double a = 0;
-            for (int l = 0; l < 3; ++l) a += Rz[3 * i + l] * c.Jinv[3 * l + j];
+            for (int l = 0; l < 3; ++l) a += Rz[3 * i + l] * body_Jinv(bd, 3 * l + j);
             T1[3 * i + j] = a;
         }
     for (int i = 0; i < 3; ++i)
@@ -353,7 +400,7 @@ __device__ inline void linearize_stage(const QpConst& c, int k, Work& w) {
                 Bf[3 * i + j] = a;
             }
         for (int i = 0; i < 9; ++i) Bv[i] = 0.0;
-        Bv[0] = Bv[4] = Bv[8] = (1.0 / c.m) * c.dt;
+        Bv[0] = Bv[4] = Bv[8] = (1.0 / body_m(bd)) * c.dt;
     } else {
         const double hatm[9] = {0, -rf[2], rf[1], rf[2], 0, -rf[0], -rf[1], rf[0], 0};
         for (int i = 0; i < 3; ++i)
@@ -363,7 +410,7 @@ __device__ inline void linearize_stage(const QpConst& c, int k, Work& w) {
                 Bf[3 * i + j] = a;
             }
         for (int i = 0; i < 3; ++i)
-            for (int j = 0; j < 3; ++j) Bv[3 * i + j] = (Rz[3 * j + i] / c.m) * c.dt;   // Rz^T / m
+            for (int j = 0; j < 3; ++j) Bv[3 * i + j] = (Rz[3 * j + i] / body_m(bd)) * c.dt;   // Rz^T / m
     }
     double* Bw = w.Bw + 18 * k;
     for (int i = 0; i < 3; ++i)
@@ -376,13 +423,15 @@ __device__ inline void linearize_stage(const QpConst& c, int k, Work& w) {
 // ------------------------------------------------------------------------------------------------
 // Condense.  Requires w.gp, w.pfw, w.xin, w.Qd, w.Rd, w.stance filled and a __syncthreads() before.
 // xref points at this hopper's window, element (k, c) at xref[(k*12 + c) * xs].
+// bd: the hopper's model body (QpConst for the scalars, or SmemBody; condense_hopper chooses).
 // Leaves H (row-major n x n, symmetric, full), g, lo, hi, fixed, cfree in place.  Returns (all threads)
 // 1 when the u-independent height rows k=0,1 are violated (SURVEY App. D2).
 // ------------------------------------------------------------------------------------------------
-__device__ inline int condense(const QpConst& c, Work& w, const double* xref, size_t xs) {
+template <class Bd>
+__device__ inline int condense(const QpConst& c, const Bd& bd, Work& w, const double* xref, size_t xs) {
     const int N = c.N, n = 6 * N, m = 11 * N, tid = threadIdx.x, T = blockDim.x;
     for (int k = tid; k < N; k += T) {
-        linearize_stage(c, k, w);
+        linearize_stage(c, bd, k, w);
         w.hinv[k] = (k >= 2) ? 1.0 / (double)(k - 1) : 0.0;
     }
     __syncthreads();
@@ -430,7 +479,7 @@ __device__ inline int condense(const QpConst& c, Work& w, const double* xref, si
     // height rows need cfree.  Exact feasibility (all-threads result): the height rows are monotone in
     // the stance fz and fz = fz_max, fx = fy = 0 satisfies every other row, so the QP is feasible iff
     // z_k(fz = fz_max on stance stages) >= z_min for k = 0..N-1 (k = 0, 1 are u-independent, App. D2).
-    const double zc = dt * dt / c.m;
+    const double zc = dt * dt / body_m(bd);
     int infeasible = 0;
     for (int k = tid; k < N; k += T) {
         double up = 0.0;
@@ -481,7 +530,7 @@ __device__ inline int condense(const QpConst& c, Work& w, const double* xref, si
             }
     }
     // gradient
-    const double ubar_alias = (c.uref_mode == 0) ? (w.stance[N - 1] ? 2.0 * c.m * c.g : 0.0) : 0.0;
+    const double ubar_alias = (c.uref_mode == 0) ? (w.stance[N - 1] ? 2.0 * body_m(bd) * c.g : 0.0) : 0.0;
     for (int a = tid; a < N; a += T) {
         double ap[3] = {0, 0, 0}, av[3] = {0, 0, 0}, aw[3] = {0, 0, 0}, at[3] = {0, 0, 0};
         const double pca = w.PC[a + 1], psa = w.PS[a + 1];
@@ -506,7 +555,7 @@ __device__ inline int condense(const QpConst& c, Work& w, const double* xref, si
             if (r < 3) v += Bva[r] * tv[0] + Bva[3 + r] * tv[1] + Bva[6 + r] * tv[2];
             v *= 2.0;
             if (r == 2 && a != N - 1) {
-                const double ub = (c.uref_mode == 0) ? ubar_alias : (w.stance[a] ? 2.0 * c.m * c.g : 0.0);
+                const double ub = (c.uref_mode == 0) ? ubar_alias : (w.stance[a] ? 2.0 * body_m(bd) * c.g : 0.0);
                 v -= 2.0 * w.Rd[2] * ub;
             }
             w.g[6 * a + r] = v;
@@ -514,6 +563,25 @@ __device__ inline int condense(const QpConst& c, Work& w, const double* xref, si
     }
     __syncthreads();
     return infeasible;
+}
+// the same with the handle's scalar body, for callers that condense without a hopper index
+__device__ inline int condense(const QpConst& c, Work& w, const double* xref, size_t xs) {
+    return condense(c, c, w, xref, xs);
+}
+// condense hopper b with its model body (QpConst::body) or, when none is set, the scalars.  Either is staged in the
+// reduction scratch w.red, which only the solvers use: one instantiation of condense, no body in registers.
+__device__ inline void stage_body(const QpConst& c, Work& w, int b, int B) {
+    for (int r = threadIdx.x; r < kBodyModel; r += blockDim.x) {
+        double v;
+        if (c.body) v = c.body[(size_t)r * B + b];
+        else v = r == 0 ? c.m : r == 1 ? c.mu : r < 5 ? c.rh[r - 2] : c.Jinv[r - 5];
+        w.red[r] = v;
+    }
+}
+__device__ inline int condense_hopper(const QpConst& c, Work& w, int b, int B, const double* xref, size_t xs) {
+    stage_body(c, w, b, B);
+    __syncthreads();
+    return condense(c, SmemBody{w.red}, w, xref, xs);
 }
 
 // algorithmic FLOP counts (FMA = 2) of the dense kernels, accumulated per hopper for the roofline report

@@ -18,7 +18,23 @@ struct SimConst {
     double m, g, h;          // mass, gravity, sim_dt
     double J[9], Jinv[9];    // row-major
     double rh[3];
+    // per-hopper plant body (hmpc_set_body_params), [kBodyPlant][B]: m, rh[3], J[9], Jinv[9]; or null: the scalars above
+    const double* body = nullptr;
 };
+constexpr int kBodyPlant = 22;        // doubles per hopper of SimConst::body
+
+// c with hopper b's plant body in place of the scalars (the simulator's m, J, Jinv, rh, robotrunner.py:37-42)
+__device__ __forceinline__ SimConst plant_body(const SimConst& c, int b, int B) {
+    SimConst s = c;
+    const double* p = c.body + b;
+    const size_t Bs = (size_t)B;
+    s.m = p[0];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) s.rh[i] = p[(1 + i) * Bs];
+#pragma unroll
+    for (int i = 0; i < 9; ++i) { s.J[i] = p[(4 + i) * Bs]; s.Jinv[i] = p[(13 + i) * Bs]; }
+    return s;
+}
 
 // (w^2 - v.v) I + 2 v v^T + 2 w hat(v): no division by |q|^2, exactly what L(q) R(q)^T gives for the
 // un-normalised quaternions that appear inside RK4 stages.

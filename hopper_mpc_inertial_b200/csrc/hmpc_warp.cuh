@@ -194,7 +194,7 @@ __device__ __forceinline__ bool wrow_coupled(const QpConst& c, const WWork& w, i
 // linearisation of one stage (gen_dt_dynamics, mpc_cvx_euler_3f.py:82-92 / 2f:82-92); one lane per stage.
 // Same arithmetic as linearize_stage (hmpc_qp.cuh); Bv is not stored: 3f  dt/m I,  2f  dt/m Rz^T (wbv).
 // ------------------------------------------------------------------------------------------------
-__device__ inline void wlinearize_stage(const QpConst& c, const double gp[4], const double pf[3], double* czk,
+__device__ inline void wlinearize_stage(const QpConst& c, const Body& bd, const double gp[4], const double pf[3], double* czk,
                                         double* szk, double* Bw) {
     double sn, cs;
     sincos(gp[3], &sn, &cs);
@@ -203,12 +203,12 @@ __device__ inline void wlinearize_stage(const QpConst& c, const double gp[4], co
     const double d[3] = {pf[0] - gp[0], pf[1] - gp[1], pf[2] - gp[2]};
     double rf[3];
     mat3_vec(Rz, d, rf);
-    rf[0] += c.rh[0]; rf[1] += c.rh[1]; rf[2] += c.rh[2];
+    rf[0] += bd.rh[0]; rf[1] += bd.rh[1]; rf[2] += bd.rh[2];
     double T1[9], Jw[9], JwRzT[9], Bf[9];
     for (int i = 0; i < 3; ++i)
         for (int j = 0; j < 3; ++j) {
             double a = 0;
-            for (int l = 0; l < 3; ++l) a += Rz[3 * i + l] * c.Jinv[3 * l + j];
+            for (int l = 0; l < 3; ++l) a += Rz[3 * i + l] * bd.Jinv[3 * l + j];
             T1[3 * i + j] = a;
         }
     for (int i = 0; i < 3; ++i)
@@ -248,24 +248,24 @@ __device__ inline void wlinearize_stage(const QpConst& c, const double gp[4], co
             Bw[6 * i + 3 + j] = JwRzT[3 * i + j] * c.dt;
         }
 }
-// dt * B[6:9, 0:3] of stage k, row-major (linearize_stage's Bv)
-__device__ __forceinline__ void wbv(const QpConst& c, const WWork& w, int k, double Bv[9]) {
-    const double s = (1.0 / c.m) * c.dt;
+// dt * B[6:9, 0:3] of stage k, row-major (linearize_stage's Bv); m = the hopper's model mass
+__device__ __forceinline__ void wbv(const QpConst& c, double m, const WWork& w, int k, double Bv[9]) {
+    const double s = (1.0 / m) * c.dt;
     if (c.dyn == 3) {
         Bv[0] = s; Bv[1] = 0; Bv[2] = 0; Bv[3] = 0; Bv[4] = s; Bv[5] = 0; Bv[6] = 0; Bv[7] = 0; Bv[8] = s;
     } else {
         const double cs = w.cz[k], sn = w.sz[k];
         // (Rz^T / m) dt with Rz = [[c, s, 0], [-s, c, 0], [0, 0, 1]]
-        Bv[0] = (cs / c.m) * c.dt; Bv[1] = (-sn / c.m) * c.dt; Bv[2] = 0;
-        Bv[3] = (sn / c.m) * c.dt; Bv[4] = (cs / c.m) * c.dt; Bv[5] = 0;
-        Bv[6] = 0; Bv[7] = 0; Bv[8] = (1.0 / c.m) * c.dt;
+        Bv[0] = (cs / m) * c.dt; Bv[1] = (-sn / m) * c.dt; Bv[2] = 0;
+        Bv[3] = (sn / m) * c.dt; Bv[4] = (cs / m) * c.dt; Bv[5] = 0;
+        Bv[6] = 0; Bv[7] = 0; Bv[8] = (1.0 / m) * c.dt;
     }
 }
 
 // Linearisation of all stages about the time-shifted previous solution: x_guess[0] = x_in, x_guess[k] = x.value[k+1]
 // (mpc_cvx_euler_3f.py:59-62; only p and yaw matter).  Needs w.xin; fills w.cz, w.sz, w.Bw (they alias the factor:
 // wcondense fills them before the first factorisation, wfinish again after the last solve).
-__device__ inline void wlinearize_all(const QpConst& c, WWork& w, int b, int B, const MpcIo& io, int lane) {
+__device__ inline void wlinearize_all(const QpConst& c, const Body& bd, WWork& w, int b, int B, const MpcIo& io, int lane) {
     const int N = c.N;
     const size_t Bs = (size_t)B;
     for (int k = lane; k < N; k += 32) {
@@ -277,7 +277,7 @@ __device__ inline void wlinearize_all(const QpConst& c, WWork& w, int b, int B, 
             gp[2] = io.Xsol[(o + 2) * Bs + b]; gp[3] = io.Xsol[(o + 5) * Bs + b];
         }
         for (int i = 0; i < 3; ++i) pf[i] = io.pf[(size_t)(3 * k + i) * Bs + b];
-        wlinearize_stage(c, gp, pf, w.cz + k, w.sz + k, w.Bw + 18 * k);
+        wlinearize_stage(c, bd, gp, pf, w.cz + k, w.sz + k, w.Bw + 18 * k);
     }
 }
 
@@ -314,11 +314,12 @@ __device__ inline void wload_sets(const QpConst& c, WWork& w, uint64_t bits, int
 __device__ inline int wcondense(const QpConst& c, WWork& w, int b, int B, const MpcIo& io, int lane) {
     const int N = c.N, n = 6 * N;
     const size_t Bs = (size_t)B;
-    // Every global load of the condensing is issued here, back to back, into registers -- state, gains, contact mask,
-    // the linearisation point and footstep of this lane's stage, this lane's reference row: ONE HBM round trip instead
-    // of four dependent ones (N <= kWarpMaxN < 32: one stage / one row per lane).
+    // Every global load of the condensing is issued here, back to back, into registers -- state, gains, model body,
+    // contact mask, the linearisation point and footstep of this lane's stage, this lane's reference row: ONE HBM round
+    // trip instead of four dependent ones (N <= kWarpMaxN < 32: one stage / one row per lane).
     const int k = lane;                                   // stage of wlinearize_all, row i = lane of the error loop
     double xq = 0.0, qq = 0.0, rq = 0.0, gp[4] = {0.0, 0.0, 0.0, 0.0}, pfq[3] = {0.0, 0.0, 0.0}, xr[12];
+    const Body bd = model_body(c, b, B);
     if (lane < 12) { xq = io.x_in[lane * Bs + b]; qq = io.Qd[lane * Bs + b]; }
     if (lane < 6) rq = io.Rd[lane * Bs + b];
     const uint64_t bits = io.Cbits[b];
@@ -338,7 +339,7 @@ __device__ inline int wcondense(const QpConst& c, WWork& w, int b, int B, const 
     if (lane < 12) { w.xin[lane] = xq; w.Qd[lane] = qq; }
     if (lane < 6) w.Rd[lane] = rq;
     wload_sets(c, w, bits, lane);
-    if (k < N) wlinearize_stage(c, gp, pfq, w.cz + k, w.sz + k, w.Bw + 18 * k);      // wlinearize_all on the loaded point
+    if (k < N) wlinearize_stage(c, bd, gp, pfq, w.cz + k, w.sz + k, w.Bw + 18 * k);      // wlinearize_all on the loaded point
     __syncwarp();
     // prefix sums of cos / sin (same summation order as condense())
     for (int i = lane; i <= N; i += 32) {
@@ -348,7 +349,7 @@ __device__ inline int wcondense(const QpConst& c, WWork& w, int b, int B, const 
     }
     __syncwarp();
     const double dt = c.dt, gdt = -c.g * dt;
-    const double zc = dt * dt / c.m;
+    const double zc = dt * dt / bd.m;
     int infeasible = 0;
     // free response + tracking error; height rows
     for (int i = lane; i <= N; i += 32) {
@@ -404,7 +405,7 @@ __device__ inline int wcondense(const QpConst& c, WWork& w, int b, int B, const 
                               dt2 * NN * w.Qd[2] + s0 * w.Qd[8]};
         const double* Bwa = w.Bw + 18 * a; const double* Bwb = w.Bw + 18 * bb;
         double Bva[9], Bvb[9];
-        wbv(c, w, a, Bva); wbv(c, w, bb, Bvb);
+        wbv(c, bd.m, w, a, Bva); wbv(c, bd.m, w, bb, Bvb);
         double MB[18];   // M3 * Bw_b (3x6)
 #pragma unroll
         for (int i = 0; i < 3; ++i)
@@ -438,7 +439,7 @@ __device__ inline int wcondense(const QpConst& c, WWork& w, int b, int B, const 
         }
     }
     // ---- gradient ----
-    const double ubar_alias = (c.uref_mode == 0) ? (w.stance[N - 1] ? 2.0 * c.m * c.g : 0.0) : 0.0;
+    const double ubar_alias = (c.uref_mode == 0) ? (w.stance[N - 1] ? 2.0 * bd.m * c.g : 0.0) : 0.0;
     for (int a = lane; a < N; a += 32) {
         double ap[3] = {0, 0, 0}, av[3] = {0, 0, 0}, aw[3] = {0, 0, 0}, at[3] = {0, 0, 0};
         const double pca = w.PC[a + 1], psa = w.PS[a + 1];
@@ -459,13 +460,13 @@ __device__ inline int wcondense(const QpConst& c, WWork& w, int b, int B, const 
         }
         const double* Bwa = w.Bw + 18 * a;
         double Bva[9];
-        wbv(c, w, a, Bva);
+        wbv(c, bd.m, w, a, Bva);
         for (int r = 0; r < 6; ++r) {
             double v = Bwa[r] * tw[0] + Bwa[6 + r] * tw[1] + Bwa[12 + r] * tw[2];
             if (r < 3) v += Bva[r] * tv[0] + Bva[3 + r] * tv[1] + Bva[6 + r] * tv[2];
             v *= 2.0;
             if (r == 2 && a != N - 1) {
-                const double ub = (c.uref_mode == 0) ? ubar_alias : (w.stance[a] ? 2.0 * c.m * c.g : 0.0);
+                const double ub = (c.uref_mode == 0) ? ubar_alias : (w.stance[a] ? 2.0 * bd.m * c.g : 0.0);
                 v -= 2.0 * w.Rd[2] * ub;
             }
             w.g[6 * a + r] = v;
@@ -942,9 +943,10 @@ __device__ inline void wprep(const QpConst& c, WWork& w, double* rec, int32_t* f
     if (lane < 12) rx[lane] = w.xin[lane];
     if (lane == 0) *flag = infeasible ? PREP_INFEASIBLE : PREP_OK;
 }
-// wfetch (solve kernel): take hopper b's record, rebuild the index sets, warm start.  Returns 0 when the hopper must
-// take the CTA kernel (no valid previous tick / infeasible height row).
-__device__ inline int wfetch(const QpConst& c, WWork& w, double* rec, const int32_t* flag, int b, int B, const MpcIo& io, int lane) {
+// wfetch (solve kernel): take hopper b's record, rebuild the index sets, warm start; mu = the hopper's friction
+// coefficient.  Returns 0 when the hopper must take the CTA kernel (no valid previous tick / infeasible height row).
+__device__ inline int wfetch(const QpConst& c, WWork& w, double& mu, double* rec, const int32_t* flag, int b, int B, const MpcIo& io,
+                             int lane) {
     const int N = c.N, n = 6 * N, m = 11 * N;
     const size_t Bs = (size_t)B;
     // Every global load of the fetch is issued here, back to back, into registers (n <= 64: two entries per lane,
@@ -955,6 +957,7 @@ __device__ inline int wfetch(const QpConst& c, WWork& w, double* rec, const int3
     const double* rx = rh + ((N + 7) & ~7);
     const int f = *flag;
     const uint64_t bits = io.Cbits[b];
+    const double mub = c.body ? c.body[Bs + b] : c.mu;     // model_body's mu, without the rest of the body
     double gq[2] = {0.0, 0.0}, uq[2] = {0.0, 0.0}, uw[2] = {0.0, 0.0};
     int8_t cq[4] = {0, 0, 0, 0}, cw[4] = {0, 0, 0, 0};
     // Warm start: stage k starts from the previous tick's stage k+1, the last two stages keep their own previous
@@ -1005,6 +1008,7 @@ __device__ inline int wfetch(const QpConst& c, WWork& w, double* rec, const int3
     const double xi = lane < 12 ? rx[lane] : 0.0;
     if (f == PREP_INVALID) { HMPC_EMUL_COUNT(4); return 0; }
     if (f == PREP_INFEASIBLE) { HMPC_EMUL_COUNT(5); return 0; }
+    mu = mub;
     w.Hc = rec;
     wload_sets(c, w, bits, lane);
 #ifndef HMPC_HOST_EMUL
@@ -1036,7 +1040,8 @@ __device__ inline void wfinish(const QpConst& c, WWork& w, int b, int B, const M
     double* xs = w.err;
     const double* u = w.xp;
     const double dt = c.dt, gdt = -c.g * dt;
-    wlinearize_all(c, w, b, B, io, lane);       // the factor overwrote cz / sz / Bw
+    const Body bd = model_body(c, b, B);
+    wlinearize_all(c, bd, w, b, B, io, lane);   // the factor overwrote cz / sz / Bw
     __syncwarp();
     if (lane < 12) xs[lane] = w.xin[lane];
     if (lane < 6) {          // velocities
@@ -1046,12 +1051,12 @@ __device__ inline void wfinish(const QpConst& c, WWork& w, int b, int B, const M
             const double* uk = u + 6 * k;
             if (q < 3) {
                 // row q of dt B[6:9, 0:3]: 3f  dt/m e_q,  2f  dt/m Rz^T (same products as rollout_solution)
-                const double sm = (1.0 / c.m) * c.dt;
+                const double sm = (1.0 / bd.m) * c.dt;
                 if (c.dyn == 3) acc += sm * uk[q];
                 else {
                     const double cs = w.cz[k], sn = w.sz[k];
-                    if (q == 0) acc += ((cs / c.m) * c.dt) * uk[0] + ((-sn / c.m) * c.dt) * uk[1];
-                    else if (q == 1) acc += ((sn / c.m) * c.dt) * uk[0] + ((cs / c.m) * c.dt) * uk[1];
+                    if (q == 0) acc += ((cs / bd.m) * c.dt) * uk[0] + ((-sn / bd.m) * c.dt) * uk[1];
+                    else if (q == 1) acc += ((sn / bd.m) * c.dt) * uk[0] + ((cs / bd.m) * c.dt) * uk[1];
                     else acc += sm * uk[2];
                 }
                 if (q == 2) acc += gdt;
@@ -1125,8 +1130,9 @@ __device__ inline void wfinish(const QpConst& c, WWork& w, int b, int B, const M
 constexpr int kDeferWarmFailed = 1 << 30;     // flag bit in a deferral-list entry
 template <int SLOTS>
 __device__ inline int mpc_hopper_warp(const QpConst& c, WWork& w, double* rec, const int32_t* flag, int kcap, int b, int B, const MpcIo& io, int lane) {
-    if (!wfetch(c, w, rec, flag, b, B, io, lane)) return 0;
-    AOp A{c.N, 6 * c.N, c.dyn == 3 ? 1 : 0, c.mu, w.stance, w.hinv};
+    double mu;
+    if (!wfetch(c, w, mu, rec, flag, b, B, io, lane)) return 0;
+    AOp A{c.N, 6 * c.N, c.dyn == 3 ? 1 : 0, mu, w.stance, w.hinv};
     WInfo info{0, c.condense_flops};
     for (int trial = 0; trial <= c.retries; ++trial) {
         const int r = wtrial<SLOTS>(c, w, A, kcap, info, lane);
@@ -1265,8 +1271,9 @@ template <int SLOTS>
 __device__ inline int mpc_hopper_warp_admm(const QpConst& c, WWork& w, double* extra, double* rec, const int32_t* flag, int kcap,
                                            int b, int B, const MpcIo& io, int lane) {
     const int N = c.N, n = 6 * N, m = 11 * N;
-    if (!wfetch(c, w, rec, flag, b, B, io, lane)) return 0;
-    AOp A{N, n, c.dyn == 3 ? 1 : 0, c.mu, w.stance, w.hinv};
+    double mu;
+    if (!wfetch(c, w, mu, rec, flag, b, B, io, lane)) return 0;
+    AOp A{N, n, c.dyn == 3 ? 1 : 0, mu, w.stance, w.hinv};
     WInfo info{0, c.condense_flops};
     double *z = extra, *y = extra + m, *rv = extra + 2 * m;
     int iters = 0;
@@ -1418,7 +1425,8 @@ mpc_warp_rounds_kernel(QpConst c, int B, int kcap, int wdoubles, double* __restr
             b = __shfl_sync(kFullMask, b, 0);
             if (b >= B) { exhausted = true; break; }
             b = work_item(c, b, B);
-            if (wfetch(c, w, prep + (size_t)b * pstride, flags + b, b, B, io, lane)) { have = true; trial = 0; info.nfac = 0; info.flops = c.condense_flops; }
+            double mu;
+            if (wfetch(c, w, mu, prep + (size_t)b * pstride, flags + b, b, B, io, lane)) { have = true; trial = 0; info.nfac = 0; info.flops = c.condense_flops; A.mu = mu; }
             else if (lane == 0) defer_list[atomicAdd(defer_cnt, 1)] = b;
         }
         if (group_all(bar_id, bar_threads, !have)) break;

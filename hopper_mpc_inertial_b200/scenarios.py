@@ -35,9 +35,44 @@ def _uniforms(seed, idx0, count, k):
     return out
 
 
+# the reference body (robotrunner.py:37-42, hmpc_default_config)
+J_REF = np.array([[76148072.89e-9, 70089.52e-9, 2067970.36e-9], [70089.52e-9, 45477183.53e-9, -87045.58e-9],
+                  [2067970.36e-9, -87045.58e-9, 76287220.47e-9]])
+RH_REF = -np.array([0.02663114, 0.04435752, 6.61082088]) / 1000
+# ranges of make_batch(body=...): mass (kg), inertia scale, friction coefficient, hip offset (m, +- per axis), and the
+# relative plant/model spread of mass and inertia
+BODY_DEFAULTS = dict(mass=(6.0, 9.0), inertia=(0.8, 1.25), mu=(0.7, 1.0), rh=0.002, mismatch=0.05)
+_BODY_KEY = 0xB0D7 << 64          # Philox key offset of the body draws: every other draw keeps its stream
+
+
+def make_bodies(B, idx0=0, seed=1234, **ranges):
+    """Per-hopper bodies of hoppers idx0 .. idx0+B-1 for BatchMpc.set_body_params.  The model (what the MPC plans
+    with) gets mass U(mass), the reference inertia times U(inertia), friction U(mu) and the reference hip offset plus
+    U(-rh, rh) per axis; the plant (what the simulator integrates) gets the model's mass and inertia each times
+    1 + U(-mismatch, mismatch), and the model's hip offset.  Ranges default to BODY_DEFAULTS.  Drawn from their own
+    Philox stream keyed by the global hopper index.  Returns (body_model, body_plant), dicts of SoA arrays:
+    model m (B,), Jinv (3,3,B), rh (3,B), mu (B,);  plant m, J, Jinv, rh."""
+    bad = set(ranges) - set(BODY_DEFAULTS)
+    if bad:
+        raise ValueError(f"unknown body ranges {sorted(bad)}; known: {sorted(BODY_DEFAULTS)}")
+    r = dict(BODY_DEFAULTS, **ranges)
+    u = _uniforms(int(seed) + _BODY_KEY, idx0, B, 8)
+    m = r["mass"][0] + (r["mass"][1] - r["mass"][0]) * u[:, 0]
+    js = r["inertia"][0] + (r["inertia"][1] - r["inertia"][0]) * u[:, 1]
+    mu = r["mu"][0] + (r["mu"][1] - r["mu"][0]) * u[:, 2]
+    rh = RH_REF[None] + r["rh"] * (2.0 * u[:, 3:6] - 1.0)
+    mp = m * (1.0 + r["mismatch"] * (2.0 * u[:, 6] - 1.0))
+    jp = js * (1.0 + r["mismatch"] * (2.0 * u[:, 7] - 1.0))
+    Jm, Jp = J_REF[None] * js[:, None, None], J_REF[None] * jp[:, None, None]
+    soa = lambda a: np.ascontiguousarray(np.moveaxis(a, 0, -1))
+    model = dict(m=m.copy(), Jinv=soa(np.linalg.inv(Jm)), rh=soa(rh), mu=mu.copy())
+    plant = dict(m=mp, J=soa(Jp), Jinv=soa(np.linalg.inv(Jp)), rh=soa(rh))
+    return model, plant
+
+
 def make_batch(B, idx0=0, seed=1234, N=10, n_ticks=100, N_run=None, mpc_factor=20, dt=1e-3, mpc_dt=0.02,
                randomize_gains=True, phase_ticks=None, t_p=None, z_base=(0.30, 0.45), gain_spread=1.25,
-               dyn="3f", perturb=0.5, speed_range=(0.2, 1.0), curve_prob=0.5, tables=True):
+               dyn="3f", perturb=0.5, speed_range=(0.2, 1.0), curve_prob=0.5, tables=True, body=None):
     """Scenario for hoppers idx0 .. idx0+B-1.
 
     Each hopper gets its own straight or curved reference (goal speed 0.2..1.0 x the reference's
@@ -47,6 +82,8 @@ def make_batch(B, idx0=0, seed=1234, N=10, n_ticks=100, N_run=None, mpc_factor=2
     reference state at that instant (perturb = 1: position +-3 cm, height -2..+3 cm, roll/pitch +-0.05 rad, yaw
     +-0.2 rad, velocity +-0.2 m/s, body rates +-0.3 rad/s; the default perturb = 0.5 halves these) -- close enough
     that the height rows stay feasible through the swing phases, as in the reference's own runs.
+    body: None (every hopper has the reference body), True (make_bodies' default ranges) or a dict of make_bodies
+    ranges: adds body_model / body_plant (make_bodies) and leaves every other output as it is.
     Returns numpy arrays in the SoA layout of include/hmpc.h:
     X0 (13,B), Qdiag (12,B), Rdiag (6,B), xref_tab, pf_tab, C_tab (uint64), pf_switch (uint8), C."""
     if t_p is None:
@@ -135,4 +172,6 @@ def make_batch(B, idx0=0, seed=1234, N=10, n_ticks=100, N_run=None, mpc_factor=2
                Rdiag=np.ascontiguousarray((R_REF[None] * gr).T), curve=curve, tick_offset=off, t_p=t_p, _x0p=x0p, _xfp=xfp,
                plan=plan)
     out.update(tabs)
+    if body is not None and body is not False:
+        out["body_model"], out["body_plant"] = make_bodies(B, idx0, seed, **({} if body is True else body))
     return out

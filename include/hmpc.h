@@ -132,6 +132,24 @@ int hmpc_synchronize(hmpc_handle* h);
  * Qdiag [12][B], Rdiag [6][B].  Defaults are the reference's values for every hopper. */
 int hmpc_set_gains(hmpc_handle* h, const double* Qdiag, const double* Rdiag);
 
+/* Per-hopper body: the arguments of Mpc(t, N, m, g, mu, Jinv, rh) (mpc_cvx_euler_3f.py:12-39) and the simulator's own
+ * m, J, Jinv, rh (robotrunner.py:37-42,76), one set per hopper instead of the config's scalars -- for domain randomisation,
+ * and for model mismatch (the MPC plans with one body while the simulator integrates another).
+ *   HMPC_BODY_MODEL  what the MPC plans with: m, Jinv, rh, mu     (linearisation, condensing, friction cones, u_ref)
+ *   HMPC_BODY_PLANT  what hmpc_rk4 / the rollouts integrate: m, J, Jinv, rh   (dynamics_ct, HMPC_GATE_DETECT's leg vector)
+ *   HMPC_BODY_BOTH   both from the same arrays
+ * m [B], J [9][B] (row-major 3x3 per hopper), Jinv [9][B], rh [3][B], mu [B], device arrays, copied (stream-ordered)
+ * into storage the handle owns.  A NULL array: that quantity takes the config's scalar for every hopper; each call
+ * replaces the whole target.  All NULL: the target goes back to the config's scalars.  J with HMPC_BODY_MODEL and mu
+ * with HMPC_BODY_PLANT have no effect and are rejected.  Nothing derives Jinv from J here: pass both.
+ * The values are checked (m > 0, mu >= 0, all finite; the call synchronises the stream): on failure HMPC_ERR_BAD_ARG,
+ * hmpc_last_error() names the first offending hopper and the handle is unchanged.  Takes effect from the next solve or
+ * rollout; warm starts stay valid (every accepted point is verified against the QP built with the new body).
+ * g, tau_max, fz_max, z_min, kf, dt and N stay per handle. */
+enum { HMPC_BODY_MODEL = 1, HMPC_BODY_PLANT = 2, HMPC_BODY_BOTH = 3 };
+int hmpc_set_body_params(hmpc_handle* h, int which, const double* m, const double* J, const double* Jinv,
+                         const double* rh, const double* mu);
+
 /* convert (robotrunner.py:19-28): X [13][B] -> x [12][B]. */
 int hmpc_convert(hmpc_handle* h, const double* X, double* x);
 
