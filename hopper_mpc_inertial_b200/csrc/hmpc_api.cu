@@ -45,6 +45,9 @@ int fail(int code, const std::string& msg) {
 }  // namespace
 
 constexpr int kOrderBuckets = 4096;     // buckets of the contact-mask counting sort (order_* kernels)
+// timing events per rollout tick: main stream 0 | solver | 1 | simulator | 2; side stream (overlapped ticks) 3 | CTA kernel
+// over the deferred hoppers | 4 | their simulator step | 5
+constexpr int kTickEvents = 6;
 
 struct hmpc_handle {
     hmpc_config cfg;
@@ -66,11 +69,21 @@ struct hmpc_handle {
     int32_t* path = nullptr;      // [B]
     int32_t* ninf = nullptr;      // [B]
     double* flops = nullptr;      // [B] algorithmic FLOPs of the solver kernel
-    int* work_ctr = nullptr;      // next hopper index handed out to the persistent CTAs
-    // optional per-kernel device timing of hmpc_rollout (hmpc_set_timing)
+    int* work_ctr = nullptr;      // [2][8] per tick parity: ticket counters and deferral count (launch_mpc)
+    // optional per-kernel device timing of hmpc_rollout (hmpc_set_timing): kTickEvents per tick
     int timing = 0;
     std::vector<cudaEvent_t> ev;
+    std::vector<uint8_t> ev_side;   // [tick] 1: the tick's deferred hoppers ran on the side stream (events 3..5 valid)
     int ev_ticks = 0;
+    // overlapped rollout schedule (DESIGN.md section 5): the deferred hoppers' CTA kernel, their simulator step and their
+    // next prep run on a second stream while the main stream simulates and condenses every other hopper
+    cudaStream_t side = nullptr;      // null: serial schedule only (no warp path, or HMPC_DEFER_SERIAL=1)
+    cudaEvent_t ev_fork = nullptr;    // main -> side: the warp kernel of the tick has finished (deferral list complete)
+    cudaEvent_t ev_join = nullptr;    // side -> main: the last side-stream work of the rollout so far
+    int32_t* defer_mark = nullptr;    // [B] number of the overlapped tick in which the hopper was last deferred
+    int seq = 0;                      // number of the next overlapped tick (handle-wide; its parity picks the buffers)
+    bool side_prep = false;           // the side stream condenses the deferred hoppers of tick seq - 1 for tick seq
+    bool warm_block = true;           // HMPC_NO_WARM_BLOCK=1 (experiment): the warp kernels gather the strided state only
     // solver launch geometry
     int mpc_threads = 128;
     int mpc_grid = 0;
@@ -95,7 +108,7 @@ struct hmpc_handle {
     double* win_pf = nullptr;     // [N+1][3][B]
     uint64_t* win_C = nullptr;    // [B]
     uint8_t* win_sw = nullptr;    // [B]
-    int* defer_list = nullptr;    // [B] hoppers the warp kernel handed to the CTA kernel this tick
+    int* defer_list = nullptr;    // [2][B] per tick parity: hoppers the warp kernel handed to the CTA kernel
     // work order of the lock-step solve kernel: hoppers grouped by contact schedule (order_* kernels)
     int* work_order = nullptr;    // [B] permutation, rebuilt every tick
     double* warm = nullptr;       // [B][warm_stride] warm blocks of the warp kernels (MpcIo::warm)
@@ -125,13 +138,16 @@ namespace hmpc {
 // ------------------------------------------------------------------------------------------------
 template <bool PLANT>
 __global__ void __launch_bounds__(128)
-sim_kernel(SimConst c, int B, double* __restrict__ X, const double* __restrict__ U,
+sim_kernel(SimConst c, int B, HopperSet hs, double* __restrict__ X, const double* __restrict__ U,
            const double* __restrict__ pfa, const double* __restrict__ pfb,
            const uint8_t* __restrict__ sw, int nsteps, double* __restrict__ xin_out,
            double* __restrict__ Xlog, double* __restrict__ Ulog, double* __restrict__ Xsteps,
            const int32_t* __restrict__ st_tick, const double* __restrict__ xref_next, SimGate gt) {
-    const int b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (b >= B) return;
+    int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (hs.list) {
+        if (b >= *hs.list_cnt) return;
+        b = hs.list[b] & kListHopperMask;
+    } else if (b >= B || (hs.mark && hs.mark[b] == hs.skip)) return;
     double Xl[13], Ul[6], pa[3], pb[3];
 #pragma unroll
     for (int i = 0; i < 13; ++i) Xl[i] = X[(size_t)i * B + b];
@@ -451,7 +467,7 @@ int hmpc_create(const hmpc_config* cfg, hmpc_handle** out) {
         (e = dalloc((void**)&h->path, B * 4)) != cudaSuccess || (e = dalloc((void**)&h->ninf, B * 4)) != cudaSuccess ||
         (e = dalloc((void**)&h->code, 11 * N * B)) != cudaSuccess || (e = dalloc((void**)&h->valid, B)) != cudaSuccess ||
         (e = dalloc((void**)&h->flops, B * 8)) != cudaSuccess || (e = dalloc((void**)&h->work_ctr, 64)) != cudaSuccess ||
-        (e = dalloc((void**)&h->defer_list, B * 4)) != cudaSuccess || (e = dalloc((void**)&h->n_defer, 4)) != cudaSuccess ||
+        (e = dalloc((void**)&h->defer_list, 2 * B * 4)) != cudaSuccess || (e = dalloc((void**)&h->n_defer, 4)) != cudaSuccess ||
         (e = dalloc((void**)&h->work_order, B * 4)) != cudaSuccess || (e = dalloc((void**)&h->order_cnt, 2 * kOrderBuckets * sizeof(int))) != cudaSuccess) {
         hmpc_destroy(h);
         return fail(HMPC_ERR_ALLOC, std::string("cudaMalloc: ") + cudaGetErrorString(e));
@@ -629,6 +645,22 @@ int hmpc_create(const hmpc_config* cfg, hmpc_handle** out) {
             h->warp_ok = true;
         }
     }
+    h->warm_block = !getenv("HMPC_NO_WARM_BLOCK");
+    // overlapped rollout schedule: a second stream, of higher priority so that the deferred hoppers' CTAs are placed
+    // first as SM slots free up; HMPC_DEFER_SERIAL=1 keeps every tick on the handle's stream (A/B runs, tests)
+    const char* serial = getenv("HMPC_DEFER_SERIAL");
+    if (h->warp_ok && !(serial && atoi(serial))) {
+        int prio_lo = 0, prio_hi = 0;
+        if ((e = cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi)) != cudaSuccess ||
+            (e = cudaStreamCreateWithPriority(&h->side, cudaStreamNonBlocking, prio_hi)) != cudaSuccess ||
+            (e = cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming)) != cudaSuccess ||
+            (e = cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming)) != cudaSuccess ||
+            (e = cudaMalloc((void**)&h->defer_mark, B * 4)) != cudaSuccess ||
+            (e = cudaMemset(h->defer_mark, 0xff, B * 4)) != cudaSuccess) {    // -1: no overlapped tick has that number
+            hmpc_destroy(h);
+            return fail(HMPC_ERR_CUDA, std::string("create (side stream): ") + cudaGetErrorString(e));
+        }
+    }
     if ((e = cudaDeviceSynchronize()) != cudaSuccess) {
         hmpc_destroy(h);
         return fail(HMPC_ERR_CUDA, std::string("create: ") + cudaGetErrorString(e));
@@ -648,8 +680,11 @@ int hmpc_destroy(hmpc_handle* h) {
     cudaFree(h->gate_glob);
     cudaFree(h->prep); cudaFree(h->prep_flag); cudaFree(h->defer_list); cudaFree(h->n_defer);
     cudaFree(h->work_order); cudaFree(h->order_cnt); cudaFree(h->warm); cudaFree(h->warm_ok);
-    cudaFree(h->body_model); cudaFree(h->body_plant); cudaFree(h->body_bad);
+    cudaFree(h->body_model); cudaFree(h->body_plant); cudaFree(h->body_bad); cudaFree(h->defer_mark);
     for (cudaEvent_t e : h->ev) cudaEventDestroy(e);
+    if (h->ev_fork) cudaEventDestroy(h->ev_fork);
+    if (h->ev_join) cudaEventDestroy(h->ev_join);
+    if (h->side) cudaStreamDestroy(h->side);
     delete h;
     return HMPC_OK;
 }
@@ -753,7 +788,7 @@ int hmpc_rk4(hmpc_handle* h, double* X, const double* U, const double* pf, int n
     if (int rc = check_handle(h)) return rc;
     if (!X || !U || !pf || nsteps < 0) return fail(HMPC_ERR_BAD_ARG, "bad argument");
     const int B = h->cfg.batch;
-    launch_sim(sim_const(h), (B + 127) / 128, h->stream, B, X, U, pf, (const double*)nullptr, (const uint8_t*)nullptr, nsteps,
+    launch_sim(sim_const(h), (B + 127) / 128, h->stream, B, hmpc::HopperSet{}, X, U, pf, (const double*)nullptr, (const uint8_t*)nullptr, nsteps,
                (double*)nullptr, (double*)nullptr, (double*)nullptr, X_steps, (const int32_t*)nullptr, (const double*)nullptr,
                hmpc::SimGate{HMPC_GATE_OFF, nullptr, nullptr, nullptr, 0, 0, 0.0});
     ++h->launches;
@@ -826,17 +861,53 @@ __global__ void order_scatter_kernel(const uint64_t* __restrict__ Cbits, int B, 
     if (b < B) order[atomicAdd(&cur[order_bucket(Cbits[b])], 1)] = b;
 }
 
-__global__ void defer_stats_kernel(const int* __restrict__ work_ctr, int32_t* __restrict__ n_defer) { *n_defer += work_ctr[1]; }
+// adds the tick's deferral count to n_defer; with mark set, also stamps every deferred hopper with the tick's number
+__global__ void defer_stats_kernel(const int* __restrict__ work_ctr, int32_t* __restrict__ n_defer, const int* __restrict__ list,
+                                   int32_t* __restrict__ mark, int seq) {
+    const int cnt = work_ctr[1];
+    if (blockIdx.x == 0 && threadIdx.x == 0) *n_defer += cnt;
+    if (mark)
+        for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < cnt; i += gridDim.x * blockDim.x) mark[list[i] & hmpc::kListHopperMask] = seq;
+}
 
-cudaError_t launch_mpc(hmpc_handle* h, const hmpc::QpConst& qc, const hmpc::MpcIo& io) {
-    cudaError_t e = cudaMemsetAsync(h->work_ctr, 0, 4 * sizeof(int), h->stream);
+// counters / deferral list of a tick: overlapped ticks alternate between two sets by the parity of their number, so
+// that the next tick's reset never touches what the CTA kernel of the previous tick still reads on the side stream
+int* tick_ctr(hmpc_handle* h, int par) { return h->work_ctr + 8 * par; }
+int* tick_list(hmpc_handle* h, int par) { return h->defer_list + (size_t)par * h->cfg.batch; }
+
+hmpc::WarpLaunch warp_launch_of(hmpc_handle* h, int par, cudaStream_t st) {
+    int* ctr = tick_ctr(h, par);
+    return hmpc::WarpLaunch{h->warp_grid, h->warp_wpc, h->warp_rounds, h->warp_group, h->warp_smem, st, h->cfg.batch, h->warp_kcap,
+                            h->warp_wdoubles, h->prep, h->pstride, h->prep_flag, ctr, tick_list(h, par), ctr + 1, h->warp_admm ? 1 : 0};
+}
+
+// the CTA kernel: every hopper (l.list null) or the deferral list of the warp kernel
+void launch_cta(hmpc_handle* h, const hmpc::MpcLaunch& l, const hmpc::QpConst& qc, const hmpc::MpcIo& io) {
+    if (6 * h->cfg.N <= 64) {
+        if (h->cfg.precision == HMPC_FP32) hmpc::mpc_launch_n10_f32(l, qc, io);
+        else if (h->cfg.solver == HMPC_SOLVER_ADMM) hmpc::mpc_launch_n10_f64_admm(l, qc, io);
+        else hmpc::mpc_launch_n10_f64(l, qc, io);
+    } else if (h->mats_in_smem) hmpc::mpc_launch_wide_smem(l, qc, io);
+    else if (h->wide_ctas == 4) hmpc::mpc_launch_wide_gmem4(l, qc, io);
+    else if (h->wide_ctas == 2) hmpc::mpc_launch_wide_gmem2(l, qc, io);
+    else hmpc::mpc_launch_wide_gmem(l, qc, io);
+    ++h->launches;
+}
+
+// One tick's solve on h->stream.  overlap (warp path only): the tick takes the buffers of parity h->seq & 1, the prep
+// kernel leaves out the hoppers the side stream condenses (h->side_prep), the warp kernel waits for those, h->ev_fork
+// marks the complete deferral list, and the CTA kernel over that list is left to the caller (rollout_impl).
+cudaError_t launch_mpc(hmpc_handle* h, const hmpc::QpConst& qc, const hmpc::MpcIo& io, bool overlap = false) {
+    const int par = overlap ? (h->seq & 1) : 0;
+    int* ctr = tick_ctr(h, par);
+    cudaError_t e = cudaMemsetAsync(ctr, 0, 4 * sizeof(int), h->stream);
     if (e != cudaSuccess) return e;
     const bool warp = h->warp_ok && hmpc::warp_path_applies(h->cfg, io.init);
     if (warp) {
-        const hmpc::WarpLaunch wl{h->warp_grid, h->warp_wpc, h->warp_rounds, h->warp_group, h->warp_smem, h->stream, h->cfg.batch, h->warp_kcap,
-                                  h->warp_wdoubles, h->prep, h->pstride, h->prep_flag, h->work_ctr, h->defer_list, h->work_ctr + 1,
-                                  h->warp_admm ? 1 : 0};
-        hmpc::prep_launch(wl, qc, io);       // natural order: no lock-step there, and neighbouring warps share sectors (measured)
+        const hmpc::WarpLaunch wl = warp_launch_of(h, par, h->stream);
+        hmpc::HopperSet ps;
+        if (overlap && h->side_prep) { ps.mark = h->defer_mark; ps.skip = h->seq - 1; }
+        hmpc::prep_launch(wl, qc, io, ps);   // natural order: no lock-step there, and neighbouring warps share sectors (measured)
         hmpc::QpConst qo = qc;
         if (h->order_on && h->warp_rounds) {
             // group the hoppers by contact schedule for the lock-step kernel (see order_count_kernel)
@@ -848,21 +919,20 @@ cudaError_t launch_mpc(hmpc_handle* h, const hmpc::QpConst& qc, const hmpc::MpcI
             h->launches += 3;
             qo.work_order = h->work_order;
         }
+        if (overlap && h->side_prep && (e = cudaStreamWaitEvent(h->stream, h->ev_join, 0)) != cudaSuccess) return e;
         hmpc::warp_launch(wl, qo, io);
-        defer_stats_kernel<<<1, 1, 0, h->stream>>>(h->work_ctr, h->n_defer);
+        if (overlap) {
+            if ((e = cudaEventRecord(h->ev_fork, h->stream)) != cudaSuccess) return e;
+            defer_stats_kernel<<<h->sm_count, 256, 0, h->stream>>>(ctr, h->n_defer, tick_list(h, par), h->defer_mark, h->seq);
+        } else {
+            defer_stats_kernel<<<1, 1, 0, h->stream>>>(ctr, h->n_defer, nullptr, nullptr, 0);
+        }
         h->launches += 3;
+        if (overlap) return cudaGetLastError();
     }
     const hmpc::MpcLaunch l{h->mpc_grid, h->mpc_threads, h->mpc_smem, h->stream, h->cfg.batch, h->sm_count, h->ws,
-                            h->work_ctr + 2, warp ? h->defer_list : nullptr, warp ? h->work_ctr + 1 : nullptr};
-    if (6 * h->cfg.N <= 64) {
-        if (h->cfg.precision == HMPC_FP32) hmpc::mpc_launch_n10_f32(l, qc, io);
-        else if (h->cfg.solver == HMPC_SOLVER_ADMM) hmpc::mpc_launch_n10_f64_admm(l, qc, io);
-        else hmpc::mpc_launch_n10_f64(l, qc, io);
-    } else if (h->mats_in_smem) hmpc::mpc_launch_wide_smem(l, qc, io);
-    else if (h->wide_ctas == 4) hmpc::mpc_launch_wide_gmem4(l, qc, io);
-    else if (h->wide_ctas == 2) hmpc::mpc_launch_wide_gmem2(l, qc, io);
-    else hmpc::mpc_launch_wide_gmem(l, qc, io);
-    ++h->launches;
+                            ctr + 2, warp ? tick_list(h, par) : nullptr, warp ? ctr + 1 : nullptr};
+    launch_cta(h, l, qc, io);
     return cudaGetLastError();
 }
 
@@ -872,7 +942,7 @@ hmpc::MpcIo make_io(hmpc_handle* h, const double* x_in, const double* x_ref, con
     hmpc::MpcIo io;
     io.x_in = x_in; io.x_ref = x_ref; io.pf = pf; io.Cbits = Cbits; io.Qd = h->Qd; io.Rd = h->Rd;
     io.Xsol = h->Xsol; io.Usol = h->Usol; io.code = h->code; io.valid = h->valid;
-    if (h->warm && !getenv("HMPC_NO_WARM_BLOCK")) {       // experiment switch: the warp kernels gather the strided state only
+    if (h->warm && h->warm_block) {
         io.warm = h->warm; io.warm_ok = h->warm_ok; io.warm_stride = hmpc::warm_stride_doubles(h->cfg.N);
     }
     io.U_out = U; io.X_out = Xsol; io.U0_out = U0;
@@ -912,11 +982,12 @@ int rollout_impl(hmpc_handle* h, bool planned, double* X, const double* xref_tab
     HMPC_CUDA(cudaMemsetAsync(h->flops, 0, B * 8, h->stream));
     HMPC_CUDA(cudaMemsetAsync(h->n_defer, 0, 4, h->stream));
     if (h->timing) {
-        while ((int)h->ev.size() < 3 * n_ticks) {
+        while ((int)h->ev.size() < kTickEvents * n_ticks) {
             cudaEvent_t e;
             HMPC_CUDA(cudaEventCreate(&e));
             h->ev.push_back(e);
         }
+        h->ev_side.assign(n_ticks, 0);
     }
     h->ev_ticks = h->timing ? n_ticks : 0;
     if (h->gate_mode == HMPC_GATE_SCHEDULE && (planned ? !h->gate_glob : !h->gate_tab))
@@ -930,19 +1001,29 @@ int rollout_impl(hmpc_handle* h, bool planned, double* X, const double* xref_tab
     hmpc::convert_kernel<<<sim_grid, 128, 0, h->stream>>>(Bi, X, h->xin);
     ++h->launches;
     if (X_log) HMPC_CUDA(cudaMemcpyAsync(X_log, X, 13 * B * 8, cudaMemcpyDeviceToDevice, h->stream));
+    // Overlapped schedule (DESIGN.md section 5): with more than one tick from the caller's tables, the CTA kernel over a
+    // warm tick's deferred hoppers, their simulator step and their next condensing run on h->side while h->stream
+    // simulates and condenses every other hopper.  The planned rollout rewrites one reference window per tick, which
+    // the side stream would still read: it keeps the serial schedule.
+    const bool overlap = h->side && !planned && n_ticks > 1;
+    h->side_prep = false;
+    bool joined = true;
     for (int t = 0; t < n_ticks; ++t) {
         const double *xr, *pf;
         const uint64_t* Cm;
         const uint8_t* sw;
+        auto table_rows = [&](int tt) {
+            const size_t row = (size_t)(tick0 + tt);
+            xr = xref_tab + row * 12 * B; pf = pf_tab + row * 3 * B; Cm = C_tab + row * B;
+            sw = pf_switch ? pf_switch + row * B : nullptr;
+        };
         if (planned) {
             hmpc::plan_rows_kernel<<<dim3(sim_grid, N + 1), 128, 0, h->stream>>>(h->plan, Bi, tick0 + t, N + 1, N + 1, h->win_xref, h->win_pf);
             hmpc::plan_masks_kernel<<<dim3(sim_grid, 1), 128, 0, h->stream>>>(h->plan, Bi, tick0 + t, 1, h->win_pf, h->win_C, h->win_sw);
             h->launches += 2;
             xr = h->win_xref; pf = h->win_pf; Cm = h->win_C; sw = h->win_sw;
         } else {
-            const size_t row = (size_t)(tick0 + t);
-            xr = xref_tab + row * 12 * B; pf = pf_tab + row * 3 * B; Cm = C_tab + row * B;
-            sw = pf_switch ? pf_switch + row * B : nullptr;
+            table_rows(t);
         }
         hmpc::SimGate gate{h->gate_mode, nullptr, nullptr, nullptr, tick0 + t, h->gate_max_tick, h->leg_max * h->leg_max};
         if (h->gate_mode == HMPC_GATE_SCHEDULE) {
@@ -950,16 +1031,52 @@ int rollout_impl(hmpc_handle* h, bool planned, double* X, const double* xref_tab
             else gate.bits = h->gate_tab + (size_t)(tick0 + t) * B;
         }
         hmpc::MpcIo io = make_io(h, h->xin, xr, pf, Cm, (init && t == 0) ? 1 : 0, 1, nullptr, nullptr, h->U0, st, it);
-        if (h->timing) HMPC_CUDA(cudaEventRecord(h->ev[3 * t], h->stream));
-        HMPC_CUDA(launch_mpc(h, qc, io));
-        if (h->timing) HMPC_CUDA(cudaEventRecord(h->ev[3 * t + 1], h->stream));
-        launch_sim(sc, sim_grid, h->stream,
-            Bi, X, (const double*)h->U0, pf, pf + 3 * B, sw, h->cfg.mpc_factor, h->xin,
-            X_log ? X_log + (size_t)(t + 1) * 13 * B : nullptr, U_log ? U_log + (size_t)t * 6 * B : nullptr,
-            (double*)nullptr, respawn ? (const int32_t*)h->st_tick : nullptr, respawn ? xr + 12 * B : nullptr, gate);
-        if (h->timing) HMPC_CUDA(cudaEventRecord(h->ev[3 * t + 2], h->stream));
-        ++h->launches;
+        const bool ov = overlap && hmpc::warp_path_applies(h->cfg, io.init);
+        cudaEvent_t* ev = h->timing ? &h->ev[(size_t)kTickEvents * t] : nullptr;
+        if (ev) HMPC_CUDA(cudaEventRecord(ev[0], h->stream));
+        HMPC_CUDA(launch_mpc(h, qc, io, ov));
+        if (ev) HMPC_CUDA(cudaEventRecord(ev[1], h->stream));
+        // sim_main: every hopper but the ones deferred in this tick (their controls are not solved yet)
+        hmpc::HopperSet main_set;
+        if (ov) { main_set.mark = h->defer_mark; main_set.skip = h->seq; }
+        auto sim = [&](cudaStream_t s, const hmpc::HopperSet& hs) {
+            launch_sim(sc, sim_grid, s,
+                Bi, hs, X, (const double*)h->U0, pf, pf + 3 * B, sw, h->cfg.mpc_factor, h->xin,
+                X_log ? X_log + (size_t)(t + 1) * 13 * B : nullptr, U_log ? U_log + (size_t)t * 6 * B : nullptr,
+                (double*)nullptr, respawn ? (const int32_t*)h->st_tick : nullptr, respawn ? xr + 12 * B : nullptr, gate);
+            ++h->launches;
+        };
+        sim(h->stream, main_set);
+        if (ev) HMPC_CUDA(cudaEventRecord(ev[2], h->stream));
+        if (!ov) continue;
+        // side stream: the deferred hoppers of this tick -- CTA kernel, simulator step, next tick's condensing.  Every
+        // kernel here reads and writes the columns of these hoppers only (per-hopper state, outputs, prep records); the
+        // CTA workspace and this parity's counters / list are not used by the main stream until it waits on ev_join.
+        const int par = h->seq & 1;
+        int* ctr = tick_ctr(h, par);
+        hmpc::HopperSet dset;
+        dset.list = tick_list(h, par); dset.list_cnt = ctr + 1;
+        HMPC_CUDA(cudaStreamWaitEvent(h->side, h->ev_fork, 0));
+        if (ev) HMPC_CUDA(cudaEventRecord(ev[3], h->side));
+        launch_cta(h, hmpc::MpcLaunch{h->mpc_grid, h->mpc_threads, h->mpc_smem, h->side, Bi, h->sm_count, h->ws, ctr + 2, dset.list, dset.list_cnt},
+                   qc, io);
+        if (ev) HMPC_CUDA(cudaEventRecord(ev[4], h->side));
+        sim(h->side, dset);
+        if (ev) { HMPC_CUDA(cudaEventRecord(ev[5], h->side)); h->ev_side[t] = 1; }
+        h->side_prep = t + 1 < n_ticks;
+        if (h->side_prep) {
+            table_rows(t + 1);
+            const hmpc::MpcIo io_next = make_io(h, h->xin, xr, pf, Cm, 0, 1, nullptr, nullptr, h->U0, st, it);
+            hmpc::prep_launch(warp_launch_of(h, par, h->side), qc, io_next, dset);
+            ++h->launches;
+        }
+        HMPC_CUDA(cudaEventRecord(h->ev_join, h->side));
+        joined = false;
+        ++h->seq;
     }
+    // the caller's stream sees the whole rollout
+    if (!joined) HMPC_CUDA(cudaStreamWaitEvent(h->stream, h->ev_join, 0));
+    h->side_prep = false;
     HMPC_CUDA(cudaGetLastError());
     return HMPC_OK;
 }
@@ -1069,14 +1186,30 @@ int hmpc_set_timing(hmpc_handle* h, int enable) {
     return HMPC_OK;
 }
 
+namespace {
+// solver and simulator device time of rollout tick t: the main-stream intervals plus, for an overlapped tick, the
+// side-stream intervals of the deferred hoppers (which overlap the next tick's main-stream work)
+int tick_time(hmpc_handle* h, int t, float* mpc, float* sim) {
+    const cudaEvent_t* ev = &h->ev[(size_t)kTickEvents * t];
+    HMPC_CUDA(cudaEventElapsedTime(mpc, ev[0], ev[1]));
+    HMPC_CUDA(cudaEventElapsedTime(sim, ev[1], ev[2]));
+    if (h->ev_side[t]) {
+        float m = 0, s = 0;
+        HMPC_CUDA(cudaEventElapsedTime(&m, ev[3], ev[4]));
+        HMPC_CUDA(cudaEventElapsedTime(&s, ev[4], ev[5]));
+        *mpc += m; *sim += s;
+    }
+    return HMPC_OK;
+}
+}  // namespace
+
 int hmpc_kernel_times(hmpc_handle* h, double* mpc_ms, double* sim_ms, int* n_ticks) {
     if (int rc = check_handle(h)) return rc;
     HMPC_CUDA(cudaStreamSynchronize(h->stream));
     double a = 0.0, b = 0.0;
     for (int t = 0; t < h->ev_ticks; ++t) {
         float m1 = 0, m2 = 0;
-        HMPC_CUDA(cudaEventElapsedTime(&m1, h->ev[3 * t], h->ev[3 * t + 1]));
-        HMPC_CUDA(cudaEventElapsedTime(&m2, h->ev[3 * t + 1], h->ev[3 * t + 2]));
+        if (int rc = tick_time(h, t, &m1, &m2)) return rc;
         a += m1; b += m2;
     }
     if (mpc_ms) *mpc_ms = a;
@@ -1091,8 +1224,7 @@ int hmpc_tick_times(hmpc_handle* h, double* mpc_ms, double* sim_ms, int cap, int
     const int n = h->ev_ticks < cap ? h->ev_ticks : cap;
     for (int t = 0; t < n; ++t) {
         float m1 = 0, m2 = 0;
-        HMPC_CUDA(cudaEventElapsedTime(&m1, h->ev[3 * t], h->ev[3 * t + 1]));
-        HMPC_CUDA(cudaEventElapsedTime(&m2, h->ev[3 * t + 1], h->ev[3 * t + 2]));
+        if (int rc = tick_time(h, t, &m1, &m2)) return rc;
         if (mpc_ms) mpc_ms[t] = m1;
         if (sim_ms) sim_ms[t] = m2;
     }

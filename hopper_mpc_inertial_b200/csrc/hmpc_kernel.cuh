@@ -101,7 +101,7 @@ struct WarpLaunch {
 };
 int prep_wdoubles(int N);
 cudaError_t prep_set_smem(int bytes);
-void prep_launch(const WarpLaunch&, const QpConst&, const MpcIo&);
+void prep_launch(const WarpLaunch&, const QpConst&, const MpcIo&, const HopperSet& = HopperSet{});
 bool warp_wpc_supported(int rounds, int wpc);
 cudaError_t warp_set_smem(int rounds, int wpc, int bytes);
 cudaError_t warp_regs(int rounds, int wpc, int* regs);

@@ -23,6 +23,19 @@ struct SimConst {
 };
 constexpr int kBodyPlant = 22;        // doubles per hopper of SimConst::body
 
+// The hoppers a one-hopper-per-thread / per-warp kernel of the rollout covers (hmpc_rollout's deferral overlap,
+// DESIGN.md section 5):
+//   list set:   the entries list[0 .. *list_cnt) of a deferral list (bit 30 of an entry is a flag for the CTA kernel);
+//   mark set:   every hopper b with mark[b] != skip, i.e. all but the hoppers deferred in the tick numbered skip;
+//   neither:    every hopper.
+struct HopperSet {
+    const int* list = nullptr;
+    const int* list_cnt = nullptr;
+    const int32_t* mark = nullptr;
+    int skip = 0;
+};
+constexpr int kListHopperMask = ~(1 << 30);
+
 // c with hopper b's plant body in place of the scalars (the simulator's m, J, Jinv, rh, robotrunner.py:37-42)
 __device__ __forceinline__ SimConst plant_body(const SimConst& c, int b, int B) {
     SimConst s = c;

@@ -1321,19 +1321,28 @@ inline bool warp_path_applies(const hmpc_config& cfg, int init) {
 #ifndef HMPC_HOST_EMUL
 // ------------------------------------------------------------------------------------------------
 // Prep kernel: one warp per hopper, plain grid.  Small per-warp slice and no factor: many warps per SM hide the HBM
-// latency of the loads and the dependent arithmetic of the condensing.
+// latency of the loads and the dependent arithmetic of the condensing.  hs: the hoppers to condense (the overlapped
+// rollout condenses the previous tick's deferred hoppers from their list on the side stream, the rest here).
 // ------------------------------------------------------------------------------------------------
 #ifndef HMPC_PREP_MINB
 #define HMPC_PREP_MINB 4
 #endif
 template <int WPC>
 __global__ void __launch_bounds__(32 * WPC, HMPC_PREP_MINB)
-mpc_prep_kernel(QpConst c, int B, int wdoubles, double* __restrict__ prep, size_t pstride, int32_t* __restrict__ flags, MpcIo io) {
+mpc_prep_kernel(QpConst c, int B, int wdoubles, double* __restrict__ prep, size_t pstride, int32_t* __restrict__ flags, HopperSet hs,
+                MpcIo io) {
     extern __shared__ double smem[];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const int ticket = blockIdx.x * WPC + wid;
-    if (ticket >= B) return;
-    const int b = work_item(c, ticket, B);
+    int b;
+    if (hs.list) {
+        if (ticket >= *hs.list_cnt) return;
+        b = hs.list[ticket] & kListHopperMask;
+    } else {
+        if (ticket >= B) return;
+        b = work_item(c, ticket, B);
+        if (hs.mark && hs.mark[b] == hs.skip) return;
+    }
     WWork w;
     wcarve(w, smem + (size_t)wid * wdoubles, c.N, kPrepKcap);
     wprep(c, w, prep + (size_t)b * pstride, flags + b, b, B, io, lane);

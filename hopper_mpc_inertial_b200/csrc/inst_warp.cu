@@ -57,10 +57,10 @@ int prep_wdoubles(int N) { return (int)warp_work_doubles(N, kPrepKcap); }
 cudaError_t prep_set_smem(int bytes) {
     return cudaFuncSetAttribute(mpc_prep_kernel<kPrepWpc>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
 }
-void prep_launch(const WarpLaunch& l, const QpConst& qc, const MpcIo& io) {
+void prep_launch(const WarpLaunch& l, const QpConst& qc, const MpcIo& io, const HopperSet& hs) {
     const int wd = prep_wdoubles(qc.N);
     mpc_prep_kernel<kPrepWpc><<<(l.B + kPrepWpc - 1) / kPrepWpc, 32 * kPrepWpc, (size_t)wd * 8 * kPrepWpc, l.stream>>>(
-        qc, l.B, wd, l.prep, l.pstride, l.flags, io);
+        qc, l.B, wd, l.prep, l.pstride, l.flags, hs, io);
 }
 
 // ADMM mode: free-running warps, one CTA per SM

@@ -12,7 +12,8 @@
  *    an array documented as [R][C][B] stores element (r,c,b) at ((r*C)+c)*B + b.
  *  - Element type is double (FP64) for every floating-point array at the boundary, whatever the
  *    internal solver precision (hmpc_config.precision).
- *  - A handle is bound to one device and one stream; calls are stream-asynchronous; a handle is
+ *  - A handle is bound to one device and one stream (a multi-tick hmpc_rollout also uses a second stream the
+ *    handle owns, joined back into the handle's stream before the call's work ends); calls are stream-asynchronous; a handle is
  *    not thread-safe.  The library allocates only its own opaque workspace.
  *  - There is no CPU fallback: creating a handle without a usable CUDA device fails.
  */
@@ -267,7 +268,10 @@ int hmpc_solve_stats(hmpc_handle* h, int32_t* nfac, int32_t* path, int32_t* n_in
 
 /* Per-kernel device timing of hmpc_rollout: when enabled, CUDA events are recorded on the handle's stream
  * around every launch.  hmpc_kernel_times synchronises the stream and returns the summed durations (ms)
- * of the solver kernel and of the simulator kernel over the most recent hmpc_rollout and its tick count. */
+ * of the solver kernel and of the simulator kernel over the most recent hmpc_rollout and its tick count.
+ * In a multi-tick rollout on the warp-per-hopper path the deferred hoppers' solver and simulator kernels run on a
+ * second stream of the handle, beside the next tick's work (DESIGN.md section 5); their own event intervals are added
+ * to the tick's solver and simulator times.  These intervals overlap: they no longer add up to the tick's duration. */
 int hmpc_set_timing(hmpc_handle* h, int enable);
 int hmpc_kernel_times(hmpc_handle* h, double* mpc_ms, double* sim_ms, int* n_ticks);
 /* The same per tick: mpc_ms / sim_ms are HOST arrays of at least cap doubles (either may be NULL); *n_ticks receives
