@@ -11,8 +11,8 @@ import subprocess
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _CSRC = os.path.join(_HERE, "csrc")
-UNITS = ["hmpc_api.cu", "inst_warp.cu", "inst_n10_f64.cu", "inst_n10_f64_admm.cu", "inst_n10_f32.cu", "inst_wide_smem.cu", "inst_wide_gmem.cu", "inst_wide_gmem2.cu", "inst_wide_gmem4.cu"]
-HEADERS = ["hmpc_qp.cuh", "hmpc_mpc.cuh", "hmpc_sim.cuh", "hmpc_kernel.cuh", "hmpc_warp.cuh", "hmpc_tile.cuh", "hmpc_plan.cuh"]
+UNITS = ["hmpc_api.cu", "inst_warp.cu", "inst_n10_f64.cu", "inst_n10_f64_admm.cu", "inst_n10_f32.cu", "inst_wide_gmem2.cu", "inst_wide_gmem4.cu"]
+HEADERS = ["hmpc_qp.cuh", "hmpc_mpc.cuh", "hmpc_sim.cuh", "hmpc_kernel.cuh", "hmpc_warp.cuh", "hmpc_tile.cuh", "hmpc_plan.cuh", "hmpc_geometry.cuh"]
 DEPS = [os.path.join(_CSRC, f) for f in UNITS + HEADERS] + [os.path.join(_HERE, "..", "include", "hmpc.h")]
 OUT = os.path.join(_HERE, "libhmpc_b200.so")
 OBJ_DIR = os.path.join(_HERE, "build")

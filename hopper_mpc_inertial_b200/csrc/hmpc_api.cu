@@ -24,6 +24,7 @@
 #include "hmpc_mpc.cuh"
 #include "hmpc_kernel.cuh"
 #include "hmpc_warp.cuh"
+#include "hmpc_geometry.cuh"
 #include "hmpc_plan.cuh"
 
 namespace {
@@ -83,21 +84,11 @@ struct hmpc_handle {
     int32_t* defer_mark = nullptr;    // [B] number of the overlapped tick in which the hopper was last deferred
     int seq = 0;                      // number of the next overlapped tick (handle-wide; its parity picks the buffers)
     bool side_prep = false;           // the side stream condenses the deferred hoppers of tick seq - 1 for tick seq
-    bool warm_block = true;           // HMPC_NO_WARM_BLOCK=1 (experiment): the warp kernels gather the strided state only
-    // solver launch geometry
-    int mpc_threads = 128;
-    int mpc_grid = 0;
-    size_t mpc_smem = 0;
-    bool mats_in_smem = false;
-    int wide_ctas = 1;               // L2-workspace kernel (long horizons): resident CTAs per SM it is compiled for
-    double* ws = nullptr;     // per-CTA matrix workspace when the matrices do not fit in shared memory
+    hmpc::Geometry geo;               // launch geometry of the CTA kernel and the warp-per-hopper kernel (hmpc_geometry.cuh)
+    double* ws = nullptr;     // per-CTA matrix workspace of the N > 10 kernels (geo.ws_bytes)
     int64_t launches = 0;
-    // warp-per-hopper warm path (hmpc_warp.cuh): geometry, per-warp Hessian workspace, deferral list
-    bool warp_ok = false;
-    bool warp_admm = false;      // solver = ADMM: the warp kernel is mpc_warp_admm_kernel
-    int warp_rounds = 0, warp_group = 0;
-    int warp_grid = 0, warp_wpc = 1, warp_kcap = 0, warp_wdoubles = 0, warp_per_sm = 0, warp_regs = 0;
-    size_t warp_smem = 0, pstride = 0;
+    // warp-per-hopper warm path (hmpc_warp.cuh)
+    size_t pstride = 0;
     double* prep = nullptr;       // [B][pstride] QP records the prep kernel hands to the solve kernel
     int32_t* prep_flag = nullptr; // [B]
     // device-side planner (hmpc_plan.cuh): global tables owned by the handle, per-hopper arrays owned by the caller
@@ -394,6 +385,27 @@ void inv3(const double* J, double* Ji) {
     Ji[6] = (d * h - e * g) / det; Ji[7] = (b * g - a * h) / det; Ji[8] = (a * e - b * d) / det;
 }
 
+// the CTA kernel builds (HMPC_CTA_BUILDS); any other id is refused and nothing is launched
+cudaError_t cta_set_smem(hmpc::CtaBuild b, int bytes) {
+    switch (b) {
+#define CALL(name, threads) case hmpc::CTA_##name: return hmpc::mpc_set_smem_##name(bytes);
+        HMPC_CTA_BUILDS(CALL)
+#undef CALL
+        default: return cudaErrorInvalidValue;
+    }
+}
+// the CTA kernel over every hopper (l.list null) or over the deferral list of the warp kernel
+cudaError_t launch_cta(hmpc_handle* h, const hmpc::MpcLaunch& l, const hmpc::QpConst& qc, const hmpc::MpcIo& io) {
+    switch (h->geo.cta) {
+#define CALL(name, threads) case hmpc::CTA_##name: hmpc::mpc_launch_##name(l, qc, io); break;
+        HMPC_CTA_BUILDS(CALL)
+#undef CALL
+        default: return cudaErrorInvalidValue;
+    }
+    ++h->launches;
+    return cudaSuccess;
+}
+
 }  // namespace
 
 extern "C" {
@@ -455,9 +467,25 @@ int hmpc_create(const hmpc_config* cfg, hmpc_handle** out) {
         if (ep != cudaSuccess) { hmpc_destroy(h); return fail(HMPC_ERR_CUDA, std::string("cudaGetDeviceProperties: ") + cudaGetErrorString(ep)); }
     }
     h->sm_count = prop.multiProcessorCount;
-    const size_t B = (size_t)cfg->batch, N = (size_t)cfg->N, n = 6 * N;
-    auto dalloc = [&](void** p, size_t bytes) { return cudaMalloc(p, bytes); };
+    // launch geometry, from the device limits and the register counts of the warp kernel builds
+    hmpc::DeviceLimits lim;
+    lim.sm_count = prop.multiProcessorCount;
+    lim.smem_block = prop.sharedMemPerBlockOptin;
+    lim.smem_sm = prop.sharedMemPerMultiprocessor;
+    lim.l2 = (size_t)prop.l2CacheSize;
     cudaError_t e = cudaSuccess;
+    if (hmpc::warp_path_applies(*cfg, 0)) {
+        if (cfg->solver == HMPC_SOLVER_ADMM)
+            for (int i = 0; i < hmpc::kNumAdmmBuilds && e == cudaSuccess; ++i) e = hmpc::warp_admm_regs(hmpc::kAdmmWpc[i], &lim.admm_regs[i]);
+        else
+            for (int i = 0; i < hmpc::kNumWarpBuilds && e == cudaSuccess; ++i) e = hmpc::warp_regs(hmpc::kWarpWpc[i], &lim.warp_regs[i]);
+        if (e != cudaSuccess) { hmpc_destroy(h); return fail(HMPC_ERR_CUDA, std::string("cudaFuncGetAttributes (warp kernel): ") + cudaGetErrorString(e)); }
+    }
+    h->geo = hmpc::launch_geometry(*cfg, hmpc::warp_kcap(*cfg), lim);
+    const hmpc::Geometry& g = h->geo;
+    if (const char* why = g.unsupported) { hmpc_destroy(h); return fail(HMPC_ERR_UNSUPPORTED, why); }
+    const size_t B = (size_t)cfg->batch, N = (size_t)cfg->N;
+    auto dalloc = [&](void** p, size_t bytes) { return cudaMalloc(p, bytes); };
     if ((e = dalloc((void**)&h->Qd, 12 * B * 8)) != cudaSuccess || (e = dalloc((void**)&h->Rd, 6 * B * 8)) != cudaSuccess ||
         (e = dalloc((void**)&h->Xsol, (N + 1) * 12 * B * 8)) != cudaSuccess ||
         (e = dalloc((void**)&h->Usol, N * 6 * B * 8)) != cudaSuccess ||
@@ -493,163 +521,40 @@ int hmpc_create(const hmpc_config* cfg, hmpc_handle** out) {
         delete[] tmp;
         if (e != cudaSuccess) { hmpc_destroy(h); return fail(HMPC_ERR_CUDA, std::string("cudaMemcpy gains: ") + cudaGetErrorString(e)); }
     }
-    // solver geometry
-    const size_t vec_bytes = ((hmpc::work_vec_doubles((int)N) + 1) & ~(size_t)1) * 8;
-    const int fsize = cfg->precision == HMPC_FP32 ? 4 : 8;
-    const size_t mat_bytes = hmpc::mat_doubles((int)N, fsize) * 8;
-    const size_t smem_cap = (size_t)prop.sharedMemPerBlockOptin;
-    h->mats_in_smem = (vec_bytes + mat_bytes + 1024 <= smem_cap);
-    // N > 10: the matrices go to the L2 workspace even when they would fit in shared memory -- two 128-register CTAs per
-    // SM beat one 223-register CTA with shared-memory matrices (N = 20, 65536 hoppers: 1.91 M vs 1.51 M steps/s,
-    // profiles/README.md); HMPC_WIDE_SMEM=1 selects the shared-memory kernel
-    if (n > 64) { const char* ev = getenv("HMPC_WIDE_SMEM"); if (!(ev && atoi(ev))) h->mats_in_smem = false; }
-    const size_t vec_bytes_ws = ((hmpc::work_vec_doubles((int)N, hmpc::mv_in_workspace((int)N)) + 1) & ~(size_t)1) * 8;
-    h->mpc_smem = h->mats_in_smem ? vec_bytes + mat_bytes : vec_bytes_ws;
-    // occupancy experiments (profiles/README.md): HMPC_SMEM_PAD=<bytes> pads the dynamic shared memory request
-    if (const char* pad = getenv("HMPC_SMEM_PAD")) h->mpc_smem += (size_t)atol(pad);
-    if (h->mpc_smem > smem_cap) { hmpc_destroy(h); return fail(HMPC_ERR_UNSUPPORTED, "horizon too large for shared memory"); }
-    h->mpc_threads = (n <= 64) ? 128 : 256;   // one CTA per SM beyond N = 10: use the wider CTA
-    // the 128-thread instantiations are compiled for shared-memory matrices only
-    if (n <= 64 && !h->mats_in_smem) { hmpc_destroy(h); return fail(HMPC_ERR_UNSUPPORTED, "shared memory too small for the N <= 10 solver kernel"); }
-    int per_sm = 1;
-    if (h->mats_in_smem) per_sm = std::max<int>(1, (int)((size_t)prop.sharedMemPerMultiprocessor / (h->mpc_smem + 1024)));
-    else {
-        // N > 10, matrices in the L2 workspace.  Three builds of the same kernel, chosen by how many CTAs the vectors
-        // in shared memory let an SM hold (HMPC_WIDE_CTAS=1|2|4 overrides; measured at 65536 hoppers, 3f,
-        // profiles/README.md): four 128-thread CTAs (128 registers; N = 20: 2.10 M steps/s), two 256-thread CTAs
-        // (128 registers; N = 20: 1.93 M, N = 40: 0.56 M), one 256-thread CTA (235 registers; N = 40: 0.42 M).
-        // More independent hoppers per SM win because each hopper's pivot chain leaves most of its warps waiting.
-        // Four CTAs per SM only while their workspaces stay L2-resident (N <= 22 on a 126 MB L2; N = 40 with four
-        // 128-thread CTAs streams its factors from HBM: 0.43 M instead of 0.56 M steps/s).
-        const size_t ws_cta = mat_bytes + hmpc::ws_mv_doubles((int)N) * 8;
-        h->wide_ctas = ((size_t)h->sm_count * 4 * ws_cta <= (size_t)prop.l2CacheSize) ? 4 : 2;
-        if (const char* ev = getenv("HMPC_WIDE_CTAS")) { const int v = atoi(ev); if (v == 1 || v == 2 || v == 4) h->wide_ctas = v; }
-        per_sm = std::max<int>(1, std::min<int>(h->wide_ctas, (int)((size_t)prop.sharedMemPerMultiprocessor / (h->mpc_smem + 1024))));
-        if (per_sm < h->wide_ctas) h->wide_ctas = per_sm >= 2 ? 2 : 1;
-        if (h->wide_ctas == 4) h->mpc_threads = 128;
-        per_sm = std::min(per_sm, h->wide_ctas);
-    }
-    h->mpc_grid = (int)std::min<size_t>(B, (size_t)h->sm_count * per_sm);
-    if (!h->mats_in_smem) {
-        if ((e = cudaMalloc((void**)&h->ws, (size_t)h->mpc_grid * (mat_bytes + hmpc::ws_mv_doubles((int)N) * 8))) != cudaSuccess) {
-            hmpc_destroy(h);
-            return fail(HMPC_ERR_ALLOC, std::string("cudaMalloc workspace: ") + cudaGetErrorString(e));
-        }
+    if (g.ws_bytes && (e = cudaMalloc((void**)&h->ws, g.ws_bytes)) != cudaSuccess) {
+        hmpc_destroy(h);
+        return fail(HMPC_ERR_ALLOC, std::string("cudaMalloc workspace: ") + cudaGetErrorString(e));
     }
     // the attribute is process-global per kernel: always the device maximum (minus room for static shared memory),
     // so that a second handle never lowers it for the first
-    const int smem_i = (int)smem_cap - 512;
-    if (6 * h->cfg.N <= 64) {
-        if (cfg->precision == HMPC_FP32) e = hmpc::mpc_set_smem_n10_f32(smem_i);
-        else e = (cfg->solver == HMPC_SOLVER_ADMM) ? hmpc::mpc_set_smem_n10_f64_admm(smem_i) : hmpc::mpc_set_smem_n10_f64(smem_i);
-    }
-    else e = h->mats_in_smem ? hmpc::mpc_set_smem_wide_smem(smem_i) : (h->wide_ctas == 4 ? hmpc::mpc_set_smem_wide_gmem4(smem_i) : h->wide_ctas == 2 ? hmpc::mpc_set_smem_wide_gmem2(smem_i) : hmpc::mpc_set_smem_wide_gmem(smem_i));
-    if (e != cudaSuccess ||
+    const int smem_i = (int)prop.sharedMemPerBlockOptin - 512;
+    if ((e = cta_set_smem(g.cta, smem_i)) != cudaSuccess ||
         (e = cudaFuncSetAttribute(hmpc::condense_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_i)) != cudaSuccess ||
         (e = cudaFuncSetAttribute(hmpc::linearize_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_i)) != cudaSuccess) {
         hmpc_destroy(h);
         return fail(HMPC_ERR_CUDA, std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(e));
     }
-    // ---- warp-per-hopper warm path: cut the SM's shared memory into per-warp slices ----
-    if (hmpc::warp_path_applies(*cfg, 0) && cfg->solver == HMPC_SOLVER_ADMM) {
-        // ADMM mode: free-running warps, one CTA per SM, as many warps as the larger slices (z, y, rho behind the
-        // exact path's slice) allow among the instantiated CTA sizes
-        h->warp_kcap = hmpc::warp_kcap(*cfg);
-        h->warp_wdoubles = (int)(hmpc::warp_work_doubles((int)N, h->warp_kcap) + hmpc::warp_admm_doubles((int)N));
-        const size_t wbytes = (size_t)h->warp_wdoubles * 8;
-        int wpc = 0;
-        for (int cand : {10, 6}) if (!wpc && hmpc::warp_admm_wpc_supported(cand) && wbytes * cand + 1024 <= smem_cap) wpc = cand;
-        if (wpc) {
-            h->warp_wpc = wpc; h->warp_per_sm = wpc; h->warp_smem = wbytes * wpc; h->warp_rounds = 0; h->warp_group = wpc;
-            h->warp_grid = (int)std::min<size_t>(((size_t)B + wpc - 1) / wpc, (size_t)h->sm_count);
-            h->pstride = hmpc::prep_stride((int)N);
-            if ((e = cudaMalloc((void**)&h->prep, B * h->pstride * 8)) != cudaSuccess ||
-                (e = cudaMalloc((void**)&h->warm, B * (size_t)hmpc::warm_stride_doubles((int)N) * 8)) != cudaSuccess ||
-                (e = cudaMalloc((void**)&h->warm_ok, B)) != cudaSuccess || (e = cudaMemset(h->warm_ok, 0, B)) != cudaSuccess ||
-                (e = cudaMalloc((void**)&h->prep_flag, B * 4)) != cudaSuccess) {
-                hmpc_destroy(h);
-                return fail(HMPC_ERR_ALLOC, std::string("cudaMalloc QP records: ") + cudaGetErrorString(e));
-            }
-            if ((e = hmpc::warp_admm_set_smem(wpc, smem_i)) != cudaSuccess || (e = hmpc::prep_set_smem(smem_i)) != cudaSuccess ||
-                (e = hmpc::warp_admm_regs(wpc, &h->warp_regs)) != cudaSuccess) {
-                hmpc_destroy(h);
-                return fail(HMPC_ERR_CUDA, std::string("cudaFuncSetAttribute (ADMM warp kernel): ") + cudaGetErrorString(e));
-            }
-            h->warp_ok = true;
-            h->warp_admm = true;
+    // warp-per-hopper warm path: QP records of the prep kernel, warm blocks
+    if (g.warp) {
+        h->pstride = hmpc::prep_stride((int)N);
+        if ((e = cudaMalloc((void**)&h->prep, B * h->pstride * 8)) != cudaSuccess ||
+            (e = cudaMalloc((void**)&h->warm, B * (size_t)hmpc::warm_stride_doubles((int)N) * 8)) != cudaSuccess ||
+            (e = cudaMalloc((void**)&h->warm_ok, B)) != cudaSuccess || (e = cudaMemset(h->warm_ok, 0, B)) != cudaSuccess ||
+            (e = cudaMalloc((void**)&h->prep_flag, B * 4)) != cudaSuccess) {
+            hmpc_destroy(h);
+            return fail(HMPC_ERR_ALLOC, std::string("cudaMalloc QP records: ") + cudaGetErrorString(e));
         }
-    } else if (hmpc::warp_path_applies(*cfg, 0)) {
-        h->warp_kcap = hmpc::warp_kcap(*cfg);
-        h->warp_wdoubles = (int)hmpc::warp_work_doubles((int)N, h->warp_kcap);
-        const size_t wbytes = (size_t)h->warp_wdoubles * 8;
-        const size_t sm_smem = (size_t)prop.sharedMemPerMultiprocessor;
-        int best_w = 0, best_wpc = 1;
-        // default: lock-step rounds, all warps of the SM in one CTA (one instruction stream per SM: measured 6 % (3f)
-        // to 20 % (2f) faster than free-running warps); HMPC_WARP_ROUNDS=0 selects the barrier-free kernel
-        int rounds = 1;
-        if (const char* ev = getenv("HMPC_WARP_ROUNDS")) rounds = atoi(ev) ? 1 : 0;
-        auto warps_for = [&](int wpc, int* regs_out) -> int {
-            int regs = 128;
-            if (hmpc::warp_regs(rounds, wpc, &regs) != cudaSuccess) { cudaGetLastError(); return 0; }
-            if (wbytes * wpc + 512 > smem_cap) return 0;
-            int ctas = (int)(sm_smem / (wbytes * wpc + 1024));
-            const int by_regs = (int)(65536 / ((size_t)((regs + 7) & ~7) * 32 * wpc));
-            ctas = std::min(std::min(ctas, by_regs), 32);
-            *regs_out = regs;
-            return ctas * wpc;
-        };
-        const int cand_free[3] = {4, 2, 1}, cand_rounds[11] = {15, 14, 13, 12, 11, 10, 8, 7, 6, 5, 4};
-        const int* cand = rounds ? cand_rounds : cand_free;
-        for (int ci = 0; ci < (rounds ? 11 : 3); ++ci) {
-            int regs = 0;
-            const int wtot = warps_for(cand[ci], &regs);
-            if (wtot > best_w) { best_w = wtot; best_wpc = cand[ci]; h->warp_regs = regs; }
-        }
-        if (const char* ev = getenv("HMPC_WARP_WPC")) {
-            const int v = atoi(ev);
-            int regs = 0;
-            if (hmpc::warp_wpc_supported(rounds, v)) { const int wtot = warps_for(v, &regs); if (wtot > 0) { best_wpc = v; best_w = wtot; h->warp_regs = regs; } }
-        }
-        if (const char* ev = getenv("HMPC_WARP_PER_SM")) {
-            const int v = atoi(ev);
-            if (v >= best_wpc && v < best_w) best_w = (v / best_wpc) * best_wpc;
-        }
-        if (best_w > 0) {
-            h->warp_wpc = best_wpc;
-            h->warp_per_sm = best_w;
-            h->warp_smem = wbytes * best_wpc;
-            const size_t want = ((size_t)B + best_wpc - 1) / best_wpc;
-            h->warp_grid = (int)std::min<size_t>(want, (size_t)h->sm_count * (best_w / best_wpc));
-            h->pstride = hmpc::prep_stride((int)N);
-            if ((e = cudaMalloc((void**)&h->prep, B * h->pstride * 8)) != cudaSuccess ||
-                (e = cudaMalloc((void**)&h->warm, B * (size_t)hmpc::warm_stride_doubles((int)N) * 8)) != cudaSuccess ||
-                (e = cudaMalloc((void**)&h->warm_ok, B)) != cudaSuccess || (e = cudaMemset(h->warm_ok, 0, B)) != cudaSuccess ||
-                (e = cudaMalloc((void**)&h->prep_flag, B * 4)) != cudaSuccess) {
-                hmpc_destroy(h);
-                return fail(HMPC_ERR_ALLOC, std::string("cudaMalloc QP records: ") + cudaGetErrorString(e));
-            }
-            h->warp_rounds = rounds;
-            if (const char* ev = getenv("HMPC_WORK_ORDER")) h->order_on = atoi(ev) ? 1 : 0;
-            // lock-step group = all warps of the CTA, one re-alignment barrier after the factorisation (measured, 131072
-            // hoppers: groups of 12 / 6 / 4 / 3 / 2 warps 8.38 / 7.83 / 7.48 / 7.30 / 7.12 M steps/s; with the barrier
-            // 8.48 M); HMPC_WARP_GROUP / HMPC_WARP_SYNCS override.  Encoded as group + 256 * barriers.
-            int grp = best_wpc, nsync = 1;
-            if (const char* ev = getenv("HMPC_WARP_GROUP")) { const int v = atoi(ev); if (v >= 1 && v <= best_wpc) grp = v; }
-            if (const char* ev = getenv("HMPC_WARP_SYNCS")) { const int v = atoi(ev); if (v >= 0 && v <= 2) nsync = v; }
-            h->warp_group = grp + 256 * nsync;
-            if ((e = hmpc::warp_set_smem(rounds, best_wpc, smem_i)) != cudaSuccess ||
-                (e = hmpc::prep_set_smem(smem_i)) != cudaSuccess) {
-                hmpc_destroy(h);
-                return fail(HMPC_ERR_CUDA, std::string("cudaFuncSetAttribute (warp kernel): ") + cudaGetErrorString(e));
-            }
-            h->warp_ok = true;
+        if ((e = g.admm ? hmpc::warp_admm_set_smem(g.wpc, smem_i) : hmpc::warp_set_smem(g.wpc, smem_i)) != cudaSuccess ||
+            (e = hmpc::prep_set_smem(smem_i)) != cudaSuccess) {
+            hmpc_destroy(h);
+            return fail(HMPC_ERR_CUDA, std::string("cudaFuncSetAttribute (warp kernel): ") + cudaGetErrorString(e));
         }
     }
-    h->warm_block = !getenv("HMPC_NO_WARM_BLOCK");
+    if (const char* ev = getenv("HMPC_WORK_ORDER")) h->order_on = atoi(ev) ? 1 : 0;
     // overlapped rollout schedule: a second stream, of higher priority so that the deferred hoppers' CTAs are placed
     // first as SM slots free up; HMPC_DEFER_SERIAL=1 keeps every tick on the handle's stream (A/B runs, tests)
     const char* serial = getenv("HMPC_DEFER_SERIAL");
-    if (h->warp_ok && !(serial && atoi(serial))) {
+    if (g.warp && !(serial && atoi(serial))) {
         int prio_lo = 0, prio_hi = 0;
         if ((e = cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi)) != cudaSuccess ||
             (e = cudaStreamCreateWithPriority(&h->side, cudaStreamNonBlocking, prio_hi)) != cudaSuccess ||
@@ -813,8 +718,8 @@ int hmpc_condense(hmpc_handle* h, const double* x_in, const double* x_guess, con
     if (int rc = check_handle(h)) return rc;
     if (!x_in || !x_guess || !x_ref || !pf || !Cbits || !H || !g || !lo || !hi)
         return fail(HMPC_ERR_BAD_ARG, "null array");
-    hmpc::condense_kernel<<<h->mpc_grid, h->mpc_threads, h->mpc_smem, h->stream>>>(
-        qp_const(h), h->cfg.batch, h->mats_in_smem ? 1 : 0, h->ws, x_in, x_guess, x_ref, pf, Cbits,
+    hmpc::condense_kernel<<<h->geo.grid, h->geo.threads, h->geo.smem, h->stream>>>(
+        qp_const(h), h->cfg.batch, h->geo.ws_bytes ? 0 : 1, h->ws, x_in, x_guess, x_ref, pf, Cbits,
         h->Qd, h->Rd, H, g, lo, hi, infeasible);
     ++h->launches;
     HMPC_CUDA(cudaGetLastError());
@@ -877,21 +782,9 @@ int* tick_list(hmpc_handle* h, int par) { return h->defer_list + (size_t)par * h
 
 hmpc::WarpLaunch warp_launch_of(hmpc_handle* h, int par, cudaStream_t st) {
     int* ctr = tick_ctr(h, par);
-    return hmpc::WarpLaunch{h->warp_grid, h->warp_wpc, h->warp_rounds, h->warp_group, h->warp_smem, st, h->cfg.batch, h->warp_kcap,
-                            h->warp_wdoubles, h->prep, h->pstride, h->prep_flag, ctr, tick_list(h, par), ctr + 1, h->warp_admm ? 1 : 0};
-}
-
-// the CTA kernel: every hopper (l.list null) or the deferral list of the warp kernel
-void launch_cta(hmpc_handle* h, const hmpc::MpcLaunch& l, const hmpc::QpConst& qc, const hmpc::MpcIo& io) {
-    if (6 * h->cfg.N <= 64) {
-        if (h->cfg.precision == HMPC_FP32) hmpc::mpc_launch_n10_f32(l, qc, io);
-        else if (h->cfg.solver == HMPC_SOLVER_ADMM) hmpc::mpc_launch_n10_f64_admm(l, qc, io);
-        else hmpc::mpc_launch_n10_f64(l, qc, io);
-    } else if (h->mats_in_smem) hmpc::mpc_launch_wide_smem(l, qc, io);
-    else if (h->wide_ctas == 4) hmpc::mpc_launch_wide_gmem4(l, qc, io);
-    else if (h->wide_ctas == 2) hmpc::mpc_launch_wide_gmem2(l, qc, io);
-    else hmpc::mpc_launch_wide_gmem(l, qc, io);
-    ++h->launches;
+    const hmpc::Geometry& g = h->geo;
+    return hmpc::WarpLaunch{g.warp_grid, g.wpc, g.group, g.warp_smem, st, h->cfg.batch, g.kcap, g.wdoubles, h->prep, h->pstride,
+                            h->prep_flag, ctr, tick_list(h, par), ctr + 1, g.admm ? 1 : 0};
 }
 
 // One tick's solve on h->stream.  overlap (warp path only): the tick takes the buffers of parity h->seq & 1, the prep
@@ -902,14 +795,14 @@ cudaError_t launch_mpc(hmpc_handle* h, const hmpc::QpConst& qc, const hmpc::MpcI
     int* ctr = tick_ctr(h, par);
     cudaError_t e = cudaMemsetAsync(ctr, 0, 4 * sizeof(int), h->stream);
     if (e != cudaSuccess) return e;
-    const bool warp = h->warp_ok && hmpc::warp_path_applies(h->cfg, io.init);
+    const bool warp = h->geo.warp && hmpc::warp_path_applies(h->cfg, io.init);
     if (warp) {
         const hmpc::WarpLaunch wl = warp_launch_of(h, par, h->stream);
         hmpc::HopperSet ps;
         if (overlap && h->side_prep) { ps.mark = h->defer_mark; ps.skip = h->seq - 1; }
         hmpc::prep_launch(wl, qc, io, ps);   // natural order: no lock-step there, and neighbouring warps share sectors (measured)
         hmpc::QpConst qo = qc;
-        if (h->order_on && h->warp_rounds) {
+        if (h->order_on && !h->geo.admm) {
             // group the hoppers by contact schedule for the lock-step kernel (see order_count_kernel)
             const int Bi = h->cfg.batch, grid = (Bi + 255) / 256;
             if ((e = cudaMemsetAsync(h->order_cnt, 0, kOrderBuckets * sizeof(int), h->stream)) != cudaSuccess) return e;
@@ -920,7 +813,7 @@ cudaError_t launch_mpc(hmpc_handle* h, const hmpc::QpConst& qc, const hmpc::MpcI
             qo.work_order = h->work_order;
         }
         if (overlap && h->side_prep && (e = cudaStreamWaitEvent(h->stream, h->ev_join, 0)) != cudaSuccess) return e;
-        hmpc::warp_launch(wl, qo, io);
+        if ((e = hmpc::warp_launch(wl, qo, io)) != cudaSuccess) return e;
         if (overlap) {
             if ((e = cudaEventRecord(h->ev_fork, h->stream)) != cudaSuccess) return e;
             defer_stats_kernel<<<h->sm_count, 256, 0, h->stream>>>(ctr, h->n_defer, tick_list(h, par), h->defer_mark, h->seq);
@@ -930,9 +823,9 @@ cudaError_t launch_mpc(hmpc_handle* h, const hmpc::QpConst& qc, const hmpc::MpcI
         h->launches += 3;
         if (overlap) return cudaGetLastError();
     }
-    const hmpc::MpcLaunch l{h->mpc_grid, h->mpc_threads, h->mpc_smem, h->stream, h->cfg.batch, h->sm_count, h->ws,
+    const hmpc::MpcLaunch l{h->geo.grid, h->geo.threads, h->geo.smem, h->stream, h->cfg.batch, h->sm_count, h->ws,
                             ctr + 2, warp ? tick_list(h, par) : nullptr, warp ? ctr + 1 : nullptr};
-    launch_cta(h, l, qc, io);
+    if ((e = launch_cta(h, l, qc, io)) != cudaSuccess) return e;
     return cudaGetLastError();
 }
 
@@ -942,7 +835,7 @@ hmpc::MpcIo make_io(hmpc_handle* h, const double* x_in, const double* x_ref, con
     hmpc::MpcIo io;
     io.x_in = x_in; io.x_ref = x_ref; io.pf = pf; io.Cbits = Cbits; io.Qd = h->Qd; io.Rd = h->Rd;
     io.Xsol = h->Xsol; io.Usol = h->Usol; io.code = h->code; io.valid = h->valid;
-    if (h->warm && h->warm_block) {
+    if (h->warm) {
         io.warm = h->warm; io.warm_ok = h->warm_ok; io.warm_stride = hmpc::warm_stride_doubles(h->cfg.N);
     }
     io.U_out = U; io.X_out = Xsol; io.U0_out = U0;
@@ -1058,8 +951,9 @@ int rollout_impl(hmpc_handle* h, bool planned, double* X, const double* xref_tab
         dset.list = tick_list(h, par); dset.list_cnt = ctr + 1;
         HMPC_CUDA(cudaStreamWaitEvent(h->side, h->ev_fork, 0));
         if (ev) HMPC_CUDA(cudaEventRecord(ev[3], h->side));
-        launch_cta(h, hmpc::MpcLaunch{h->mpc_grid, h->mpc_threads, h->mpc_smem, h->side, Bi, h->sm_count, h->ws, ctr + 2, dset.list, dset.list_cnt},
-                   qc, io);
+        HMPC_CUDA(launch_cta(h, hmpc::MpcLaunch{h->geo.grid, h->geo.threads, h->geo.smem, h->side, Bi, h->sm_count, h->ws, ctr + 2,
+                                                dset.list, dset.list_cnt},
+                             qc, io));
         if (ev) HMPC_CUDA(cudaEventRecord(ev[4], h->side));
         sim(h->side, dset);
         if (ev) { HMPC_CUDA(cudaEventRecord(ev[5], h->side)); h->ev_side[t] = 1; }
@@ -1244,9 +1138,9 @@ int hmpc_solve_stats(hmpc_handle* h, int32_t* nfac, int32_t* path, int32_t* n_in
 
 int hmpc_hot_path_info(hmpc_handle* h, int* warps_per_sm, int* kcap, int* regs, int64_t* n_deferred) {
     if (int rc = check_handle(h)) return rc;
-    if (warps_per_sm) *warps_per_sm = h->warp_ok ? h->warp_per_sm : 0;
-    if (kcap) *kcap = h->warp_ok ? h->warp_kcap : 0;
-    if (regs) *regs = h->warp_ok ? h->warp_regs : 0;
+    if (warps_per_sm) *warps_per_sm = h->geo.warp ? h->geo.warp_per_sm : 0;
+    if (kcap) *kcap = h->geo.warp ? h->geo.kcap : 0;
+    if (regs) *regs = h->geo.warp ? h->geo.regs : 0;
     if (n_deferred) {
         int32_t v = 0;
         HMPC_CUDA(cudaMemcpyAsync(&v, h->n_defer, 4, cudaMemcpyDeviceToHost, h->stream));

@@ -76,20 +76,17 @@ cudaError_t mpc_set_smem_n10_f64_admm(int bytes); // the same with the ADMM bran
 void mpc_launch_n10_f64_admm(const MpcLaunch&, const QpConst&, const MpcIo&);
 cudaError_t mpc_set_smem_n10_f32(int bytes);      // 128 threads, 5 CTAs/SM, shared-memory matrices, FP32 factor
 void mpc_launch_n10_f32(const MpcLaunch&, const QpConst&, const MpcIo&);
-cudaError_t mpc_set_smem_wide_smem(int bytes);    // 256 threads, 1 CTA/SM, shared-memory matrices, FP64 factor
-void mpc_launch_wide_smem(const MpcLaunch&, const QpConst&, const MpcIo&);
-cudaError_t mpc_set_smem_wide_gmem(int bytes);    // 256 threads, matrices in the L2-resident workspace, FP64 factor
-void mpc_launch_wide_gmem(const MpcLaunch&, const QpConst&, const MpcIo&);
-cudaError_t mpc_set_smem_wide_gmem2(int bytes);   // the same compiled for 2 CTAs/SM (<= 128 registers)
+cudaError_t mpc_set_smem_wide_gmem2(int bytes);   // 256 threads, 2 CTAs/SM (<= 128 registers), matrices in the L2-resident workspace
 void mpc_launch_wide_gmem2(const MpcLaunch&, const QpConst&, const MpcIo&);
 cudaError_t mpc_set_smem_wide_gmem4(int bytes);   // 128 threads, 4 CTAs/SM, matrices in the L2 workspace
 void mpc_launch_wide_gmem4(const MpcLaunch&, const QpConst&, const MpcIo&);
 
 
-// the warp-per-hopper warm-path kernel (hmpc_warp.cuh, instantiated in inst_warp.cu)
+// the warp-per-hopper warm-path kernel (hmpc_warp.cuh, instantiated in inst_warp.cu); the functions taking a wpc
+// return cudaErrorInvalidValue for a wpc that has no build
 struct WarpLaunch {
-    int grid, wpc, rounds;  // CTAs, warps per CTA, 1: lock-step rounds kernel
-    int group;              // rounds kernel: warps per lock-step group (named barrier)
+    int grid, wpc;          // CTAs, warps per CTA
+    int group;              // lock-step kernel: warps per lock-step group (named barrier) + 256 * re-alignment barriers
     size_t smem;            // dynamic shared memory per CTA
     cudaStream_t stream;
     int B, kcap, wdoubles;
@@ -102,11 +99,9 @@ struct WarpLaunch {
 int prep_wdoubles(int N);
 cudaError_t prep_set_smem(int bytes);
 void prep_launch(const WarpLaunch&, const QpConst&, const MpcIo&, const HopperSet& = HopperSet{});
-bool warp_wpc_supported(int rounds, int wpc);
-cudaError_t warp_set_smem(int rounds, int wpc, int bytes);
-cudaError_t warp_regs(int rounds, int wpc, int* regs);
-void warp_launch(const WarpLaunch&, const QpConst&, const MpcIo&);
-bool warp_admm_wpc_supported(int wpc);
+cudaError_t warp_set_smem(int wpc, int bytes);
+cudaError_t warp_regs(int wpc, int* regs);
+cudaError_t warp_launch(const WarpLaunch&, const QpConst&, const MpcIo&);
 cudaError_t warp_admm_set_smem(int wpc, int bytes);
 cudaError_t warp_admm_regs(int wpc, int* regs);
 

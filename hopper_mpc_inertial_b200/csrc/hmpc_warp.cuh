@@ -580,37 +580,6 @@ __device__ inline int wfactor(const QpConst& c, WWork& w, const AOp& A, int nF, 
     const double mv0 = (8 * Jb + 2 * t < nF) ? 1.0 : 0.0, mv1 = (8 * Jb + 2 * t + 1 < nF) ? 1.0 : 0.0;
     const bool ondiag0 = (2 * t == g), ondiag1 = (2 * t + 1 == g);
     int bad = 0;
-#ifdef HMPC_BULK_GATHER
-    // Hessian block of K, gathered up front: tile (I, J) of the variable rows is written where V(I, J) will live (each
-    // lane its own two entries), eight tiles -- sixteen L2 loads per lane -- in flight at a time, instead of one
-    // gather per tile inside the elimination (ncu: a third of the kernel's long-scoreboard stalls).  Entries outside the
-    // variable block (i or j >= nF) are written as 0 and produced by the elimination loop as before.
-    {
-        const int ntv = (nF + 7) >> 3, ntiles = ntv * (ntv + 1) / 2;
-        int I = 0, J = 0;
-#pragma unroll 1
-        for (int base = 0; base < ntiles; base += 8) {
-            d2 v[8];
-#pragma unroll
-            for (int u = 0; u < 8; ++u) {
-                v[u] = d2{0.0, 0.0};
-                if (base + u < ntiles) {
-                    const int i = 8 * I + g, j0 = 8 * J + 2 * t;
-                    if (i < nF) {
-                        const int ri = (int)w.idx[i];
-                        if (j0 < nF) v[u].x = w.Hc[(int)w.idx[j0] * w.ld + ri];
-                        if (j0 + 1 < nF) v[u].y = w.Hc[(int)w.idx[j0 + 1] * w.ld + ri];
-                    }
-                    if (++J > I) { ++I; J = 0; }
-                }
-            }
-#pragma unroll
-            for (int u = 0; u < 8; ++u)
-                if (base + u < ntiles) st2(L + 64 * (base + u) + fo, v[u].x, v[u].y);
-        }
-        __syncwarp();
-    }
-#endif
 #pragma unroll 1
     for (int J = 0; J < nt; ++J) {
         const int j0 = 8 * J + 2 * t;
@@ -630,11 +599,7 @@ __device__ inline int wfactor(const QpConst& c, WWork& w, const AOp& A, int nF, 
             double k0, k1;
             if (8 * I + 8 <= nF) {                                   // variables x variables (H is stored symmetric)
                 const int ri = (int)w.idx[i];
-#ifdef HMPC_BULK_GATHER
-                { const d2 kk = ld2(L + tile_off(I, J) + fo); k0 = kk.x; k1 = kk.y; }
-#else
                 k0 = hc0[ri]; k1 = hc1[ri];
-#endif
                 if (ADMM) {                                          // ADMM operator (i >= j0, j0 + 1 may exceed i: unused)
                     k0 += wweights(w, A, ri, (int)w.idx[j0]);
                     k1 += wweights(w, A, ri, (int)w.idx[j0 + 1]);
@@ -647,12 +612,7 @@ __device__ inline int wfactor(const QpConst& c, WWork& w, const AOp& A, int nF, 
                 const int ri = (int)w.idx[i];
                 const bool v0 = j0 < nF, v1 = j0 + 1 < nF;
                 const int cj0 = v0 ? (int)w.idx[j0] : 0, cj1 = v1 ? (int)w.idx[j0 + 1] : 0;
-#ifdef HMPC_BULK_GATHER
-                const d2 kk = ld2(L + tile_off(I, J) + fo);
-                const double h0 = kk.x, h1 = kk.y;
-#else
                 const double h0 = w.Hc[cj0 * w.ld + ri], h1 = w.Hc[cj1 * w.ld + ri];
-#endif
                 k0 = v0 ? h0 : 0.0; k1 = v1 ? h1 : 0.0;
                 if (ADMM) {
                     if (v0) k0 += wweights(w, A, ri, cj0);
@@ -1126,7 +1086,8 @@ __device__ inline void wfinish(const QpConst& c, WWork& w, int b, int B, const M
 }
 // Returns 1: done;  0: not attempted (no valid previous tick / infeasible height row / system larger than kcap): the
 // CTA kernel runs its whole solver;  -1: the active-set refinement itself gave up: the CTA kernel goes straight to
-// its interior point (same QP, same verified polish afterwards).
+// its interior point (same QP, same verified polish afterwards).  No kernel calls it: it is the serial statement of
+// the lock-step kernel's per-hopper loop, which the test emulation (tests/emul, tests/emul_body) runs.
 constexpr int kDeferWarmFailed = 1 << 30;     // flag bit in a deferral-list entry
 template <int SLOTS>
 __device__ inline int mpc_hopper_warp(const QpConst& c, WWork& w, double* rec, const int32_t* flag, int kcap, int b, int B, const MpcIo& io, int lane) {
@@ -1324,11 +1285,8 @@ inline bool warp_path_applies(const hmpc_config& cfg, int init) {
 // latency of the loads and the dependent arithmetic of the condensing.  hs: the hoppers to condense (the overlapped
 // rollout condenses the previous tick's deferred hoppers from their list on the side stream, the rest here).
 // ------------------------------------------------------------------------------------------------
-#ifndef HMPC_PREP_MINB
-#define HMPC_PREP_MINB 4
-#endif
 template <int WPC>
-__global__ void __launch_bounds__(32 * WPC, HMPC_PREP_MINB)
+__global__ void __launch_bounds__(32 * WPC, 4)
 mpc_prep_kernel(QpConst c, int B, int wdoubles, double* __restrict__ prep, size_t pstride, int32_t* __restrict__ flags, HopperSet hs,
                 MpcIo io) {
     extern __shared__ double smem[];
@@ -1348,34 +1306,9 @@ mpc_prep_kernel(QpConst c, int B, int wdoubles, double* __restrict__ prep, size_
     wprep(c, w, prep + (size_t)b * pstride, flags + b, b, B, io, lane);
 }
 
-// ------------------------------------------------------------------------------------------------
-// Solve kernel, free-running form: WPC independent warps per CTA, hoppers handed out one at a time (the solve times
-// differ).  Deferred hoppers are appended to defer_list.
-// ------------------------------------------------------------------------------------------------
-template <int SLOTS, int WPC, int MIN_CTAS>
-__global__ void __launch_bounds__(32 * WPC, MIN_CTAS)
-mpc_warp_kernel(QpConst c, int B, int kcap, int wdoubles, double* __restrict__ prep, size_t pstride,
-                const int32_t* __restrict__ flags, int* __restrict__ work_ctr, int* __restrict__ defer_list,
-                int* __restrict__ defer_cnt, int /*group: rounds kernel only*/, MpcIo io) {
-    extern __shared__ double smem[];
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    WWork w;
-    wcarve(w, smem + (size_t)wid * wdoubles, c.N, kcap);
-    for (;;) {
-        int b = 0;
-        if (lane == 0) b = atomicAdd(work_ctr, 1);
-        b = __shfl_sync(kFullMask, b, 0);
-        if (b >= B) break;
-        b = work_item(c, b, B);
-        const int done = mpc_hopper_warp<SLOTS>(c, w, prep + (size_t)b * pstride, flags + b, kcap, b, B, io, lane);
-        __syncwarp();
-        if (done <= 0 && lane == 0) defer_list[atomicAdd(defer_cnt, 1)] = b | (done < 0 ? kDeferWarmFailed : 0);
-    }
-}
-
-// ADMM mode (hmpc_config.solver = HMPC_SOLVER_ADMM): WPC free-running warps per CTA, one hopper each, the same ticket
-// counter and deferral list as above.  The iteration count differs from hopper to hopper by design (early exit), so
-// there is nothing to run in lock-step.
+// ADMM mode (hmpc_config.solver = HMPC_SOLVER_ADMM): WPC free-running warps per CTA, one hopper each, hoppers handed
+// out one at a time from a ticket counter, the ones it cannot finish appended to a deferral list.  The iteration
+// count differs from hopper to hopper by design (early exit), so there is nothing to run in lock-step.
 template <int WPC>
 __global__ void __launch_bounds__(32 * WPC, 1)
 mpc_warp_admm_kernel(QpConst c, int B, int kcap, int wdoubles, double* __restrict__ prep, size_t pstride,
@@ -1399,7 +1332,7 @@ mpc_warp_admm_kernel(QpConst c, int B, int kcap, int wdoubles, double* __restric
     }
 }
 
-// Lock-step form (default): the WPC warps of a CTA still own one hopper each, but start every active-set trial
+// Exact solver, lock-step form: the WPC warps of a CTA still own one hopper each, but start every active-set trial
 // together (one CTA barrier per round), so that the warps sharing an SM execute the same code at the same time and
 // share its instruction fetches.  A warp whose hopper is finished stores it and fetches the next record; since the
 // condensing moved to the prep kernel a round is one trial for every warp.

@@ -11,7 +11,8 @@ _ROOT = os.path.dirname(os.path.dirname(_HERE))
 _SO = os.path.join(_HERE, "libhmpc_emul.so")
 _DEPS = [os.path.join(_HERE, "emul.cpp"), os.path.join(_HERE, "fake_cuda", "cuda_runtime.h"),
          os.path.join(_ROOT, "include", "hmpc.h")] + \
-        [os.path.join(_ROOT, "hopper_mpc_inertial_b200", "csrc", f) for f in ("hmpc_sim.cuh", "hmpc_qp.cuh", "hmpc_mpc.cuh", "hmpc_warp.cuh", "hmpc_plan.cuh")]
+        [os.path.join(_ROOT, "hopper_mpc_inertial_b200", "csrc", f) for f in ("hmpc_sim.cuh", "hmpc_qp.cuh", "hmpc_mpc.cuh", "hmpc_warp.cuh", "hmpc_plan.cuh",
+                                                                             "hmpc_geometry.cuh")]
 _lib = None
 
 
@@ -143,6 +144,32 @@ class EmulMpc:
                                _p(np.ascontiguousarray(pfb, float)), _p(sw), int(gate_mode), _p(bits), float(leg_max))
         assert rc == 0
         return X
+
+
+GEOMETRY_FIELDS = ("unsupported", "cta", "threads", "grid", "smem", "ws_bytes", "warp", "admm", "wpc", "kcap", "wdoubles",
+                   "warp_grid", "warp_per_sm", "regs", "group", "warp_smem")
+CTA_BUILDS = ("n10_f64", "n10_f64_admm", "n10_f32", "wide_gmem4", "wide_gmem2")     # enum CtaBuild (hmpc_geometry.cuh)
+
+
+def launch_geometry(cfg, kcap, sm_count, smem_block, smem_sm, l2, warp_regs, admm_regs):
+    """hmpc_create's launch geometry (csrc/hmpc_geometry.cuh) as a dict; cta is the name of the CTA build."""
+    lib = load()
+    lib.emul_launch_geometry.argtypes = [C.c_void_p, C.c_int, C.c_int] + [C.c_longlong] * 3 + [C.c_void_p] * 3
+    wr = np.ascontiguousarray(warp_regs, np.int32)
+    ar = np.ascontiguousarray(admm_regs, np.int32)
+    out = np.zeros(16, np.int64)
+    lib.emul_launch_geometry(C.byref(cfg), int(kcap), int(sm_count), int(smem_block), int(smem_sm), int(l2), _p(wr), _p(ar), _p(out))
+    g = dict(zip(GEOMETRY_FIELDS, (int(v) for v in out)))
+    g["cta"] = CTA_BUILDS[g["cta"]]
+    return g
+
+
+def kernel_builds():
+    """The kernel build lists of csrc/hmpc_geometry.cuh: warp wpc, ADMM warp wpc, CTA build -> threads."""
+    n = np.zeros(3, np.int32)
+    w, a, t = (np.zeros(16, np.int32) for _ in range(3))
+    load().emul_kernel_builds(_p(n), _p(w), _p(a), _p(t))
+    return dict(warp=w[:n[0]].tolist(), admm=a[:n[1]].tolist(), cta=dict(zip(CTA_BUILDS, t[:n[2]].tolist())))
 
 
 def plan_tables(x0, xf, curve, off, gt, N, n_ticks, tick0=0, mpc_factor=20, dt=1e-3):

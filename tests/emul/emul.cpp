@@ -15,6 +15,7 @@
 #include "../../hopper_mpc_inertial_b200/csrc/hmpc_sim.cuh"
 #include "../../hopper_mpc_inertial_b200/csrc/hmpc_mpc.cuh"
 #include "../../hopper_mpc_inertial_b200/csrc/hmpc_warp.cuh"
+#include "../../hopper_mpc_inertial_b200/csrc/hmpc_geometry.cuh"
 #include "../../hopper_mpc_inertial_b200/csrc/hmpc_plan.cuh"
 
 using namespace hmpc;
@@ -191,6 +192,28 @@ int emul_warp_done(void) { return g_emul_warp_done; }
 // event counters of the warp emulation since the last reset ([0] = DMMA lane-calls)
 void emul_counters(long long* out, int reset) {
     for (int i = 0; i < 8; ++i) { out[i] = hmpc_emul_count[i]; if (reset) hmpc_emul_count[i] = 0; }
+}
+
+// launch geometry of hmpc_create (hmpc_geometry.cuh) for the given device limits and warp-build register counts (in
+// the order of kWarpWpc / kAdmmWpc).  out[16]: unsupported (0/1), cta, threads, grid, smem, ws_bytes, warp, admm, wpc,
+// kcap, wdoubles, warp_grid, warp_per_sm, regs, group, warp_smem.
+void emul_launch_geometry(const hmpc_config* cfg, int kcap, int sm_count, long long smem_block, long long smem_sm, long long l2,
+                          const int* warp_regs, const int* admm_regs, long long* out) {
+    DeviceLimits d;
+    d.sm_count = sm_count; d.smem_block = (size_t)smem_block; d.smem_sm = (size_t)smem_sm; d.l2 = (size_t)l2;
+    for (int i = 0; i < kNumWarpBuilds; ++i) d.warp_regs[i] = warp_regs[i];
+    for (int i = 0; i < kNumAdmmBuilds; ++i) d.admm_regs[i] = admm_regs[i];
+    const Geometry g = launch_geometry(*cfg, kcap, d);
+    const long long v[16] = {g.unsupported ? 1 : 0, g.cta, g.threads, g.grid, (long long)g.smem, (long long)g.ws_bytes, g.warp, g.admm,
+                             g.wpc, g.kcap, g.wdoubles, g.warp_grid, g.warp_per_sm, g.regs, g.group, (long long)g.warp_smem};
+    for (int i = 0; i < 16; ++i) out[i] = v[i];
+}
+// the kernel build lists: n[3] = sizes; warp_wpc, admm_wpc, cta_threads (at least 16 entries each)
+void emul_kernel_builds(int* n, int* warp_wpc, int* admm_wpc, int* cta_threads) {
+    n[0] = kNumWarpBuilds; n[1] = kNumAdmmBuilds; n[2] = kNumCtaBuilds;
+    for (int i = 0; i < kNumWarpBuilds; ++i) warp_wpc[i] = kWarpWpc[i];
+    for (int i = 0; i < kNumAdmmBuilds; ++i) admm_wpc[i] = kAdmmWpc[i];
+    for (int i = 0; i < kNumCtaBuilds; ++i) cta_threads[i] = kCtaThreads[i];
 }
 
 // condense only: H [n][n][B], g [n][B], lo/hi [m][B], infeasible [B]

@@ -82,8 +82,8 @@ def test_linearise_and_condense_against_reference_golden(dyn):
 def test_mpcontrol_matches_oracle_optimum(dyn, N, B):
     """Per-step QP solutions within 1e-5 abs + 1e-4 rel of the exact optimum (FP64), first call (two solves)
     and a warm-started second call.  Horizons cover every kernel instantiation: 128-thread shared-memory
-    (N <= 10, incl. the short horizons 3 and 5 and odd batch sizes), 256-thread shared-memory (12, 20) and the
-    global-workspace path (40, 60)."""
+    (N <= 10, incl. the short horizons 3 and 5 and odd batch sizes) and the L2-workspace builds with four (12, 20)
+    and two (40, 60) CTAs per SM."""
     sc = scenarios.make_batch(B, N=N, n_ticks=3, seed=13, dyn=dyn)
     bm = mk(B, dyn, N)
     bm.set_gains(T(sc["Qdiag"]), T(sc["Rdiag"]))

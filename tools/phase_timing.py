@@ -29,11 +29,21 @@ args = (T(sc["xref_tab"]), T(sc["pf_tab"]), T(np.ascontiguousarray(sc["C_tab"]).
 bm.rollout(X, *args, 0, W, True)
 torch.cuda.synchronize()
 lib = _lib.load() if hasattr(_lib, "load") else C.CDLL(_lib.LIB_PATH)
-buf = (C.c_ulonglong * 16)()
-fname = "hmpc_debug_phases" if N <= 10 else ("hmpc_debug_phases_wide_smem" if N <= 20 else "hmpc_debug_phases_wide_gmem")
-has = hasattr(lib, fname)
-if has:
-    getattr(lib, fname)(buf)
+# one hook per CTA-kernel unit that has one; every read resets, so the sum is the handle's build
+hooks = [getattr(lib, f) for f in ("hmpc_debug_phases", "hmpc_debug_phases_wide_gmem4", "hmpc_debug_phases_wide_gmem2") if hasattr(lib, f)]
+has = bool(hooks)
+
+
+def read_phases():
+    tot = np.zeros(16, np.uint64)
+    for f in hooks:
+        b = (C.c_ulonglong * 16)()
+        f(b)
+        tot += np.array(b[:], np.uint64)
+    return tot
+
+
+read_phases()
 t0 = time.perf_counter()
 bm.rollout(X, *args, W, K, False)
 torch.cuda.synchronize()
@@ -42,7 +52,7 @@ print(f"{B * K / dt / 1e6:.3f} M steps/s ({dt / K * 1e3:.2f} ms per tick)")
 nf, path, ninf = bm.solve_stats()
 print("factorisations per tick", float(nf.double().mean()) / K)
 if has:
-    getattr(lib, fname)(buf)
+    buf = read_phases()
     names = ["whole hopper", "load + lin. point", "condense", "solve_exact (all)", "factor", "solve (1 rhs)", "refinement loop (incl. its solves)",
              "verify_active_set", "interior point (incl. its factor/solve)", "rollout", "tiled factor: entry gather (warp 0)", "tiled factor: tile products (warp 0)", "tiled factor: diagonal tiles"]
     tot = buf[0] or 1
